@@ -2,6 +2,7 @@
 """Headline benchmark: ORCA agent-steps/sec (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config cfg2|cfg3|cfg4|cfg5]
+                  [--dump-outputs DIR]
 
 Workloads = BASELINE.json configs, one GPU's share each (env instances are independent, so N GPUs
 each own one share: weak scaling, no data-path collective; episode statistics are all-reduced
@@ -28,6 +29,10 @@ config: the expensive mid-episode phase), then W warm-up steps, then exactly K t
                 host->device and the new state comes device->host inside the timed region
   roofline      algorithmic HBM bytes / kernel time vs. the measured copy bandwidth
   cpu_baseline  the CPU oracle (restatement of RVO2, oracle/) on this box's host cores
+
+--dump-outputs DIR writes what the last timed step left for its caller (rank 0's share: positions,
+velocities and the per-agent / per-env results of the step) as DIR/<name>.npy, so that two builds
+can be compared output for output on identical seeded inputs.
 """
 from __future__ import annotations
 
@@ -40,6 +45,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from
 
 METRIC = "orca_agent_steps_per_sec"
 UNIT = "agent-steps/s"
@@ -310,6 +316,36 @@ class GpuWorkload:
     def goal_tensor(self):
         return self.alan.goal if self.alan is not None else self.st["goal"]
 
+    def outputs(self):
+        """What a caller holds after a step: the new state and the results the step wrote."""
+        out = {"pos": self.sim.pos, "vel": self.sim.vel}
+        if self.alan is not None:
+            a = self.alan
+            out.update(reward=a.reward, action_ids=a.action_ids, agent_done=a.agents_done, arrival_time=a.agents_time,
+                       env_step=a.env_step, env_done_cnt=a.env_done_cnt)
+        else:
+            out.update({k: self.st[k] for k in ("agent_done", "arrival_time", "env_step", "env_done_cnt")})
+        return out
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(wl, out_dir):
+    """DIR/<name>.npy of wl.outputs(): float32 as computed, flags as float32 and counters as float64
+    (both exact)."""
+    import numpy as np
+    arrays = {}
+    for name, t in wl.outputs().items():
+        a = t.cpu().numpy()
+        arrays[name] = a.astype(np.float32 if a.dtype in (np.float32, np.uint8) else np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
 
 def run_ours(args, cfg_name, cfg):
     import torch
@@ -359,6 +395,8 @@ def run_ours(args, cfg_name, cfg):
         barrier()
         wall = time.perf_counter() - wall0
     launches = sim.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl, args.dump_outputs)
     kernel_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]
     total_ms = sum(kernel_ms)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
@@ -560,7 +598,11 @@ def main():
                     help="episode step the (untimed) fast-forward stops at before warm-up; default per config")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-phase-profile", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     cfg = CONFIGS[args.config]
     if args.episode_step is None:
         args.episode_step = cfg["episode_step"]

@@ -5,9 +5,9 @@ do around ``sim.doStep()``; every function cites the lines it follows.  The simu
 it is the CPU oracle (``oracle.rvo2_oracle.PyRVOSimulator``), reached through the same scalar
 per-agent calls the reference makes.
 
-  env  = /root/reference/collision_avoidance/envs/collision_avoidence_env.py
-  ALAN = /root/reference/collision_avoidance/ALAN/ALAN_true.py
-  util = /root/reference/collision_avoidance/envs/utils.py
+  env  = collision_avoidance/envs/collision_avoidence_env.py   (paths in the reference project)
+  ALAN = collision_avoidance/ALAN/ALAN_true.py
+  util = collision_avoidance/envs/utils.py
 
 Pinning: ``line_intersection`` / ``comp_laser`` below are checked against golden vectors
 produced by importing the reference's own ``utils.py`` (tests/golden/make_laser_golden.py).

@@ -7,7 +7,7 @@ collision_avoidance/ALAN/ALAN_true.py:5-6), none of which exist here (SURVEY F2,
 puts inert stand-ins into ``sys.modules`` and binds ``rvo2.PyRVOSimulator`` to whatever
 PyRVOSimulator-compatible class the caller passes (the CPU oracle, a recording proxy, or
 ``collision_avoidance_b200.rvo2_compat`` on a GPU box).  Nothing in the reference is edited:
-it is imported from /root/reference as it lies.
+it is imported as it lies from the checkout named by ``$COLLISION_AVOIDANCE_REFERENCE``.
 """
 from __future__ import annotations
 
@@ -20,12 +20,13 @@ import types
 
 import numpy as np
 
-REFERENCE_ROOT = "/root/reference"
+# a checkout of the reference project (navallo/collision_avoidance); the repository does not vendor it
+REFERENCE_ROOT = os.environ.get("COLLISION_AVOIDANCE_REFERENCE", "")
 REGISTRY = {}          # gym.envs.registration.register(id=..., entry_point=...) calls seen
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "collision_avoidance"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "collision_avoidance"))
 
 
 class _Widget:

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Generates the committed golden fixtures from the REFERENCE ITSELF (run in the build
-container, where /root/reference exists; the fixtures travel, the reference does not).
+"""Generates the committed golden fixtures from the REFERENCE ITSELF (run with
+COLLISION_AVOIDANCE_REFERENCE naming a checkout of it; the fixtures are committed, the reference
+is not).
 
   laser_golden.npz   inputs + outputs of the reference's own utils.comp_laser /
                      utils.line_intersection (collision_avoidance/envs/utils.py:5-113)
@@ -15,7 +16,7 @@ from math import cos, pi, sin
 
 import numpy as np
 
-REF = "/root/reference/collision_avoidance"
+REF = os.path.join(os.environ.get("COLLISION_AVOIDANCE_REFERENCE", ""), "collision_avoidance")
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Golden fixtures recorded from the UNMODIFIED reference shells (run in the build container,
-where /root/reference exists; the fixtures travel to the GPU box, the reference does not).
+"""Golden fixtures recorded from the UNMODIFIED reference shells (run with
+COLLISION_AVOIDANCE_REFERENCE naming a checkout of the reference; the fixtures are committed, the
+reference is not).
 
 What runs: collision_avoidance/ALAN/ALAN_true.py (``Collision_Avoidance_Sim``: ``_init_world_*``
 :175-457, ``run_sim`` :106-131, ``online_step`` :569-628, ``orca_step`` :631-636, ``done_test``
@@ -43,7 +44,7 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 import _ref_stubs  # noqa: E402
 from oracle import rvo2_oracle  # noqa: E402
 
-ACT_DIR = "/root/reference/collision_avoidance/ALAN"
+ACT_DIR = os.path.join(_ref_stubs.REFERENCE_ROOT, "collision_avoidance", "ALAN")
 
 # (scenario, numAgents, action file or None = the default 8 actions, seed, recorded steps)
 ALAN_RUNS = [

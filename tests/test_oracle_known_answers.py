@@ -1,5 +1,5 @@
 """Pins the CPU oracle: analytic known answers (SURVEY T0), the reference's own golden vectors
-for the laser path (generated from /root/reference/collision_avoidance/envs/utils.py by
+for the laser path (generated from the reference's collision_avoidance/envs/utils.py by
 tests/golden/make_golden.py) and the reference's action-table fixtures."""
 import json
 import os
