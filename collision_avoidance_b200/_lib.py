@@ -33,7 +33,7 @@ MAX_ACTIONS = 16
 
 # every symbol include/orca_b200.h declares (tests check the .so exports all of them)
 EXPORTED_SYMBOLS = (
-    "orca_abi_version", "orca_last_error", "orca_create", "orca_destroy", "orca_get_params",
+    "orca_abi_version", "orca_last_error", "orca_create", "orca_destroy", "orca_get_params", "orca_set_agent_params",
     "orca_set_obstacles", "orca_obstacle_vertex_count", "orca_get_obstacle_vertices",
     "orca_step", "orca_env_step", "orca_env_step_many", "orca_neighbors", "orca_observe", "orca_step_host", "orca_step_host_ex", "orca_policy_mlp", "orca_policy_mlp_fp32", "orca_launch_count",
 )
@@ -127,6 +127,7 @@ def load() -> ctypes.CDLL:
     L.orca_create.argtypes = [ctypes.POINTER(OrcaParams), i, i, i, ctypes.POINTER(hp)]
     L.orca_destroy.argtypes = [hp]
     L.orca_get_params.argtypes = [hp, ctypes.POINTER(OrcaParams), ctypes.POINTER(i), ctypes.POINTER(i)]
+    L.orca_set_agent_params.argtypes = [hp, _vp, _vp, _vp, _vp, _vp, _vp]
     L.orca_set_obstacles.argtypes = [hp, _vp, _vp, i, _vp]
     L.orca_obstacle_vertex_count.argtypes = [hp, i]
     L.orca_get_obstacle_vertices.argtypes = [hp, i, _vp, _vp, _vp, _vp]

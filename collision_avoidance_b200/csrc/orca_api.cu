@@ -111,6 +111,11 @@ struct OrcaSim {
   int tune_calls = 0;
   double tune_ms[2] = {0.0, 0.0};  // [direct, staged]
   float* d_nbr_hint = nullptr;  // [E*N] per-agent starting threshold of the neighbor search (see agent_front)
+  // per-agent parameters (orca_set_agent_params): [E*N][2] records (orca::AgentParams, packed), or
+  // nullptr (uniform), and the largest neighbor distance and obstacle range (tho * vmax + r) among them
+  float4* d_agent_params = nullptr;
+  float max_nd = 0.f, max_orange = 0.f;
+  float cull_range = 0.f;  // obstacle range the obstacle-free maps were built for
   // uniform-grid scratch (large worlds)
   orca::GridScratch grid;
   int64_t launches = 0;
@@ -176,7 +181,7 @@ void fill_common(const OrcaSim* s, orca::StepArgs* a) {
   a->cull_geo = s->d_cull_geo;
 }
 
-template <int K, bool KFULL, int POLICY, int OL>
+template <int K, bool KFULL, int POLICY, int OL, bool HETERO = false>
 int launch_small_kpo(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
   const int N = s->N;
   // 256-thread blocks: whole envs per block (256 / N of them); measured faster than 128 / 64 / 32
@@ -194,15 +199,17 @@ int launch_small_kpo(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
   args.world_slots = (slots > 0 && slots <= 256) ? slots : 0;
   // worlds of more than 32 agents: candidates come from an in-block uniform grid (cell = neighborDist + 0.1 %)
   args.tile_grid_inv_cell = 0.f;
-  if (N > 32 && s->p.neighbor_dist > 0.f && std::getenv("ORCA_B200_NO_TILE_GRID") == nullptr)
-    args.tile_grid_inv_cell = 1.0f / (s->p.neighbor_dist * 1.001f);
-  size_t smem = orca::step_smem_bytes(K, tpb, true, args.world_slots, OL);
-  auto kern = orca::step_small_kernel<K, KFULL, POLICY, OL>;
+  // (per-agent parameters: the largest neighborDist of the table)
+  const float nd = HETERO ? s->max_nd : s->p.neighbor_dist;
+  if (N > 32 && nd > 0.f && std::getenv("ORCA_B200_NO_TILE_GRID") == nullptr)
+    args.tile_grid_inv_cell = 1.0f / (nd * 1.001f);
+  size_t smem = orca::step_smem_bytes(K, tpb, true, args.world_slots, OL, HETERO);
+  auto kern = orca::step_small_kernel<K, KFULL, POLICY, OL, HETERO>;
   // function attributes are per device: one flag per (instantiation, device)
   // (distinct handles may be driven from distinct threads: atomic flags; setting the attribute twice is harmless)
   static std::atomic<bool> attr_set[orca::kMaxDevices];
   if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
-    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)orca::step_smem_bytes(K, 256, true, 256, OL)));
+    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)orca::step_smem_bytes(K, 256, true, 256, OL, HETERO)));
     // the whole unified L1 as shared memory: the resident-block count is what this kernel lives on
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
     if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
@@ -214,7 +221,7 @@ int launch_small_kpo(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
       CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
   }
-  kern<<<blocks, tpb, smem, st>>>(args);
+  kern<<<blocks, tpb, smem, st>>>(args, HETERO ? s->d_agent_params : nullptr);
   CUDA_TRY(cudaGetLastError());
   s->launches += 1;
   return ORCA_OK;
@@ -249,6 +256,32 @@ int launch_small_k(OrcaSim* s, const orca::StepArgs& a, int policy, cudaStream_t
   }
 }
 
+// Per-agent parameters: the HETERO variants of the full tile kernel and of the grid kernel, K from the
+// handle's maxNeighbors (the width of the neighbor-list rows), lists of KFULL = false (per-agent k <= K).
+template <int K, int POLICY>
+int launch_hetero_kp(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
+  if (s->N >= s->grid_min_agents)
+    return orca::launch_grid_kpo<K, false, POLICY, ORCA_MAX_OBST_LINES, true>(s->grid, a, st, &s->launches, &g_last_error,
+                                                                              s->d_agent_params);
+  return launch_small_kpo<K, false, POLICY, ORCA_MAX_OBST_LINES, true>(s, a, st);
+}
+
+template <int K>
+int launch_hetero_k(OrcaSim* s, const orca::StepArgs& a, int policy, cudaStream_t st) {
+  switch (policy) {
+    case ORCA_POLICY_EXTERNAL:
+      return launch_hetero_kp<K, orca::POLICY_EXTERNAL>(s, a, st);
+    case ORCA_POLICY_GOAL:
+      return launch_hetero_kp<K, orca::POLICY_GOAL>(s, a, st);
+    case ORCA_POLICY_RL:
+      return launch_hetero_kp<K, orca::POLICY_RL>(s, a, st);
+    case ORCA_POLICY_ALAN:
+      return launch_hetero_kp<K, orca::POLICY_ALAN>(s, a, st);
+    default:
+      return fail(ORCA_ERR_INVALID, "unknown policy %d", policy);
+  }
+}
+
 int launch_step(OrcaSim* s, const orca::StepArgs& a0, int policy, cudaStream_t st) {
   orca::StepArgs a = a0;
   // searches that run on a shrinking threshold (worlds of more than 32 agents) start from last step's
@@ -256,6 +289,13 @@ int launch_step(OrcaSim* s, const orca::StepArgs& a0, int policy, cudaStream_t s
   if (s->d_nbr_hint != nullptr && !a.neighbors_only && std::getenv("ORCA_B200_NO_NBR_HINT") == nullptr) {
     a.nbr_hint = s->d_nbr_hint;  // allocated by orca_create (never inside a launch: the host path captures graphs)
     a.hint_slack = 2.5f * s->p.max_speed * s->p.time_step + 1e-4f;
+  }
+  if (s->d_agent_params != nullptr) {
+    a.nd_sq = s->max_nd * s->max_nd;  // what the kernels still read of it: the cell size of the uniform grid
+    const int K = pick_k(s->p.max_neighbors);
+    if (K == 5) return launch_hetero_k<5>(s, a, policy, st);
+    if (K == 10) return launch_hetero_k<10>(s, a, policy, st);
+    return launch_hetero_k<16>(s, a, policy, st);
   }
   if (s->N >= s->grid_min_agents) {
     return orca::launch_grid_step(s->grid, a, policy, st, &s->launches, &g_last_error);
@@ -265,6 +305,37 @@ int launch_step(OrcaSim* s, const orca::StepArgs& a0, int policy, cudaStream_t s
   if (k == 10) return launch_small_k<10, true>(s, a, policy, st);
   if (k <= 16) return launch_small_k<16, false>(s, a, policy, st);
   return fail(ORCA_ERR_UNSUPPORTED, "max_neighbors=%d > 16 is not supported", k);
+}
+
+// The largest obstacle range (timeHorizonObst * maxSpeed + radius) of any agent of the handle.
+float obstacle_range(const OrcaSim* s) {
+  if (s->d_agent_params != nullptr) return s->max_orange;
+  return s->p.time_horizon_obst * s->p.max_speed + s->p.radius;
+}
+
+// Obstacle-free maps of the current obstacle worlds for the current obstacle range: where no edge can
+// come within that range, the step skips the BSP walk.
+int build_cull_maps(OrcaSim* s) {
+  cudaFree(s->d_cull_rows);
+  cudaFree(s->d_cull_geo);
+  s->d_cull_rows = nullptr;
+  s->d_cull_geo = nullptr;
+  if (s->vert_stride == 0 || std::getenv("ORCA_B200_NO_OBST_CULL") != nullptr) return ORCA_OK;
+  const float orange = obstacle_range(s);
+  const size_t n_worlds = s->worlds.size();
+  std::vector<uint32_t> rows(n_worlds * orca_host::kCullGrid);
+  std::vector<float4> geo(n_worlds);
+  for (size_t w = 0; w < n_worlds; ++w) {
+    const orca_host::CullMap M = orca_host::build_cull_map(s->worlds[w], orange);
+    std::memcpy(&rows[w * orca_host::kCullGrid], M.rows, sizeof(M.rows));
+    geo[w] = make_float4(M.x0, M.y0, M.inv_cx, M.inv_cy);
+  }
+  CUDA_TRY(cudaMalloc(&s->d_cull_rows, rows.size() * sizeof(uint32_t)));
+  CUDA_TRY(cudaMalloc(&s->d_cull_geo, geo.size() * sizeof(float4)));
+  CUDA_TRY(cudaMemcpy(s->d_cull_rows, rows.data(), rows.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(s->d_cull_geo, geo.data(), geo.size() * sizeof(float4), cudaMemcpyHostToDevice));
+  s->cull_range = orange;
+  return ORCA_OK;
 }
 
 int ensure_host_staging(OrcaSim* s) {
@@ -332,6 +403,7 @@ int orca_destroy(OrcaSim* s) {
   cudaFree(s->d_vel);
   cudaFree(s->d_aux);
   cudaFree(s->d_nbr_hint);
+  cudaFree(s->d_agent_params);
   if (s->host_graph_exec) cudaGraphExecDestroy(s->host_graph_exec);
   for (int c = 0; c < kHostChunksMax; ++c) {
     if (s->host_streams[c]) cudaStreamDestroy(s->host_streams[c]);
@@ -423,21 +495,57 @@ int orca_set_obstacles(OrcaSim* s, const float* xy, const int32_t* poly_sizes, i
   }
   s->shared_nodes = s->per_env ? 0 : nodes[0];
   s->vert_stride = stride;
-  // obstacle-free maps: where no edge can come within the obstacle range, the step skips the BSP walk
-  if (std::getenv("ORCA_B200_NO_OBST_CULL") == nullptr) {
-    const float orange = s->p.time_horizon_obst * s->p.max_speed + s->p.radius;
-    std::vector<uint32_t> rows((size_t)n_worlds * orca_host::kCullGrid);
-    std::vector<float4> geo((size_t)n_worlds);
-    for (int w = 0; w < n_worlds; ++w) {
-      const orca_host::CullMap M = orca_host::build_cull_map(s->worlds[(size_t)w], orange);
-      std::memcpy(&rows[(size_t)w * orca_host::kCullGrid], M.rows, sizeof(M.rows));
-      geo[(size_t)w] = make_float4(M.x0, M.y0, M.inv_cx, M.inv_cy);
+  return build_cull_maps(s);
+}
+
+int orca_set_agent_params(OrcaSim* s, const float* neighbor_dist, const int32_t* max_neighbors, const float* time_horizon,
+                          const float* time_horizon_obst, const float* radius, const float* max_speed) {
+  if (s == nullptr) return fail(ORCA_ERR_INVALID, "null handle");
+  const bool any = neighbor_dist || max_neighbors || time_horizon || time_horizon_obst || radius || max_speed;
+  const size_t n = (size_t)s->E * s->N;
+  std::vector<float4> table;
+  float max_nd = 0.f, max_orange = 0.f;
+  if (any) {
+    table.resize(2 * n);
+    for (size_t i = 0; i < n; ++i) {
+      const float nd = neighbor_dist ? neighbor_dist[i] : s->p.neighbor_dist;
+      const int k = max_neighbors ? max_neighbors[i] : s->p.max_neighbors;
+      const float th = time_horizon ? time_horizon[i] : s->p.time_horizon;
+      const float tho = time_horizon_obst ? time_horizon_obst[i] : s->p.time_horizon_obst;
+      const float r = radius ? radius[i] : s->p.radius;
+      const float vmax = max_speed ? max_speed[i] : s->p.max_speed;
+      if (!std::isfinite(nd) || !std::isfinite(th) || !std::isfinite(tho) || !std::isfinite(r) || !std::isfinite(vmax))
+        return fail(ORCA_ERR_INVALID, "agent %zu: parameters must be finite", i);
+      if (!(th > 0.f) || !(tho > 0.f)) return fail(ORCA_ERR_INVALID, "agent %zu: time_horizon and time_horizon_obst must be > 0", i);
+      if (!(nd >= 0.f) || !(r >= 0.f) || !(vmax >= 0.f))
+        return fail(ORCA_ERR_INVALID, "agent %zu: neighbor_dist, radius and max_speed must be >= 0", i);
+      if (k < 0 || k > s->p.max_neighbors)
+        return fail(ORCA_ERR_INVALID, "agent %zu: max_neighbors %d outside [0, %d] (the handle's max_neighbors)", i, k,
+                    s->p.max_neighbors);
+      // the expressions of fill_common: a table of the handle's values gives the uniform results bit for bit
+      const float orange = tho * vmax + r;
+      table[2 * i] = make_float4(r, vmax, 1.0f / th, 1.0f / tho);
+      table[2 * i + 1] = make_float4(nd * nd, orange * orange, orca::bits_to_float(k), 0.f);
+      max_nd = std::max(max_nd, nd);
+      max_orange = std::max(max_orange, orange);
     }
-    CUDA_TRY(cudaMalloc(&s->d_cull_rows, rows.size() * sizeof(uint32_t)));
-    CUDA_TRY(cudaMalloc(&s->d_cull_geo, geo.size() * sizeof(float4)));
-    CUDA_TRY(cudaMemcpy(s->d_cull_rows, rows.data(), rows.size() * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(s->d_cull_geo, geo.data(), geo.size() * sizeof(float4), cudaMemcpyHostToDevice));
   }
+  DeviceGuard guard(s->device);
+  CUDA_TRY(cudaDeviceSynchronize());  // steps in flight may still read the old table
+  if (s->host_graph_exec) {  // the captured host step has the old table baked into its kernel arguments
+    cudaGraphExecDestroy(s->host_graph_exec);
+    s->host_graph_exec = nullptr;
+  }
+  cudaFree(s->d_agent_params);
+  s->d_agent_params = nullptr;
+  if (any) {
+    CUDA_TRY(cudaMalloc(&s->d_agent_params, table.size() * sizeof(float4)));
+    CUDA_TRY(cudaMemcpy(s->d_agent_params, table.data(), table.size() * sizeof(float4), cudaMemcpyHostToDevice));
+    s->max_nd = max_nd;
+    s->max_orange = max_orange;
+  }
+  // the obstacle-free maps must cover the largest obstacle range of any agent
+  if (s->vert_stride > 0 && obstacle_range(s) != s->cull_range) return build_cull_maps(s);
   return ORCA_OK;
 }
 

@@ -217,6 +217,9 @@ struct GridSource {
   ORCA_HD float2 pos(int q) const { return ORCA_LDG(reinterpret_cast<const float2*>(&spv[q])); }
   ORCA_HD float2 vel(int q) const { return ORCA_LDG(reinterpret_cast<const float2*>(&spv[q]) + 1); }
   ORCA_HD int local_id(int q) const { return ORCA_LDG(&orig[q]) - env_n0; }
+  // per-agent records (orca_set_agent_params' table, HETERO kernels only): the radius by original id
+  const float4* params = nullptr;
+  ORCA_HD float radius(int q) const { return ORCA_LDG(&params[2 * (size_t)ORCA_LDG(&orig[q])]).x; }
 };
 
 #if defined(__CUDACC__)
@@ -481,12 +484,14 @@ __global__ void __launch_bounds__(256) grid_scatter_kernel(const float2* __restr
 // warp's agents share cells (coherent candidate loops, cache-friendly reads).
 // OL: obstacle-line slots per agent, as in step_small_kernel: the K + 2 variant (worlds of at most 4
 // obstacle vertices) fits 1024 instead of 768 threads per SM.
-template <int K, bool KFULL, int POLICY, int OL = ORCA_MAX_OBST_LINES>
+// HETERO: per-agent parameters (agent_front), neighbor radii gathered from the records by original id.
+template <int K, bool KFULL, int POLICY, int OL = ORCA_MAX_OBST_LINES, bool HETERO = false>
 __global__ void __launch_bounds__(ORCA_GRID_TPB, (OL <= 2 ? 1024 : 768) / ORCA_GRID_TPB) step_grid_kernel(const StepArgs a, const float4* __restrict__ spv,
                                                            const int* __restrict__ sidx,
                                                            const int* __restrict__ cell_start,
                                                            const GridParams* __restrict__ gpp,
-                                                           const int* __restrict__ env_step_snap) {
+                                                           const int* __restrict__ env_step_snap,
+                                                           const float4* __restrict__ agent_params) {
   extern __shared__ float4 smem4[];
   const int tpb = blockDim.x;
   float4* s_lines = smem4;
@@ -495,6 +500,7 @@ __global__ void __launch_bounds__(ORCA_GRID_TPB, (OL <= 2 ? 1024 : 768) / ORCA_G
   int* s_meta = reinterpret_cast<int*>(s_nv + tpb);
   int* s_warp_cnt = s_meta + tpb;
   unsigned char* s_queue = reinterpret_cast<unsigned char*>(s_warp_cnt + 8);
+  float* s_vmax = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(s_queue + tpb) + 15) & ~(uintptr_t)15);
   const int T = a.E * a.N;
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   const bool valid = j < T;
@@ -516,7 +522,8 @@ __global__ void __launch_bounds__(ORCA_GRID_TPB, (OL <= 2 ? 1024 : 768) / ORCA_G
     env_live = env_step_snap[a.E + env] < a.N;
     GridSource src;
     src.spv = spv;
-    src.full_range_sq = a.nd_sq;
+    src.full_range_sq = HETERO ? ORCA_LDG(&agent_params[2 * (size_t)g + 1]).x : a.nd_sq;
+    if (HETERO) src.params = agent_params;
     src.orig = sidx;
     src.cell_start = cell_start;
     src.gp = *gpp;
@@ -531,10 +538,12 @@ __global__ void __launch_bounds__(ORCA_GRID_TPB, (OL <= 2 ? 1024 : 768) / ORCA_G
     c.v = v2(pv.z, pv.w);
     if (!a.neighbors_only) c.aim = (POLICY == POLICY_EXTERNAL) ? a.pref[g] : a.goal[g];
     const ObstacleWorld W = global_world_with_cull(a, env);
-    alive = agent_front<K, KFULL, POLICY, OL>(a, env, g, estep, src, W, L, warp_mask, c);
+    alive = agent_front<K, KFULL, POLICY, OL, HETERO>(a, env, g, estep, src, W, L, warp_mask, c, agent_params);
+    if (HETERO) s_vmax[threadIdx.x] = ORCA_LDG(&agent_params[2 * (size_t)g]).y;
   }
   if (a.neighbors_only) return;  // uniform over the grid
-  block_lp3<K>(s_lines, s_pool, s_meta, s_nv, s_queue, s_warp_cnt, alive && !c.overflow && c.fail < c.n, c, a.vmax);
+  block_lp3<K, HETERO>(s_lines, s_pool, s_meta, s_nv, s_queue, s_warp_cnt, alive && !c.overflow && c.fail < c.n, c, a.vmax, false,
+                       s_vmax);
   const unsigned slow_mask = __ballot_sync(0xffffffffu, alive && c.overflow);
   if (!alive) return;
   c.nv = s_nv[threadIdx.x];
@@ -552,7 +561,9 @@ __global__ void __launch_bounds__(ORCA_GRID_TPB, (OL <= 2 ? 1024 : 768) / ORCA_G
     again.env = env;
     again.env_n0 = env * a.N;
     again.self = j;
-    apply_slow_result(agent_slow_path<K, KFULL>(slow_params(a), again, global_world(a, env), L, K + OL, slow_mask, c.p, c.v, c.pref), c);
+    if (HETERO) again.params = agent_params;
+    apply_slow_result(agent_slow_path<K, KFULL, GridSource, HETERO>(HETERO ? slow_params(a, agent_params, g) : slow_params(a), again, global_world(a, env), L,
+                                                                    K + OL, slow_mask, c.p, c.v, c.pref), c);
   }
   agent_back<POLICY>(a, env, la, g, estep, c, env_live);
 }
@@ -605,8 +616,9 @@ inline int grid_ensure(GridScratch& G, const StepArgs& a, cudaStream_t st, std::
 
 constexpr int kGridLaunchesPerStep = 5;  // G1 bounds, G2 count, G3 scan, G4 scatter, G5 step
 
-template <int K, bool KFULL, int POLICY, int OL>
-int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t* launches, std::string* err) {
+template <int K, bool KFULL, int POLICY, int OL, bool HETERO = false>
+int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t* launches, std::string* err,
+                    const float4* agent_params = nullptr) {
   const int T = a.E * a.N;
   const int rc = grid_ensure(G, a, st, err);
   if (rc != 0) return rc;
@@ -624,8 +636,8 @@ int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t*
   StepArgs args = a;
   // the step kernel only READS the step counters in this path, from the copy G2 made
   const int stpb = ORCA_GRID_TPB;
-  const size_t smem = step_smem_bytes(K, stpb, false, 0, OL);
-  auto kern = step_grid_kernel<K, KFULL, POLICY, OL>;
+  const size_t smem = step_smem_bytes(K, stpb, false, 0, OL, HETERO);
+  auto kern = step_grid_kernel<K, KFULL, POLICY, OL, HETERO>;
   int dev = 0;
   ORCA_GRID_TRY(cudaGetDevice(&dev));
   // function attributes are per device; setting one is idempotent, so a racing second thread is harmless
@@ -636,7 +648,7 @@ int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t*
     if (dev < kMaxDevices) attr_set[dev].store(true, std::memory_order_release);
   }
   args.grid_path = 1;
-  kern<<<(T + stpb - 1) / stpb, stpb, smem, st>>>(args, G.sorted_pv, G.sorted_idx, G.cell_start, G.params, G.env_step_snap);
+  kern<<<(T + stpb - 1) / stpb, stpb, smem, st>>>(args, G.sorted_pv, G.sorted_idx, G.cell_start, G.params, G.env_step_snap, agent_params);
   ORCA_GRID_TRY(cudaGetLastError());
   *launches += kGridLaunchesPerStep;
   return 0;

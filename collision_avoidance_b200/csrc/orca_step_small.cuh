@@ -105,6 +105,28 @@ struct StepArgs {
   const float4* cull_geo;
 };
 
+// Per-agent ORCA parameters (orca_set_agent_params), read by the HETERO kernels only, from a table that
+// travels next to StepArgs (whose scalars stay the handle's values): two float4 per agent,
+// {radius, maxSpeed, 1 / timeHorizon, 1 / timeHorizonObst} and {neighborDist^2, obstacle range^2,
+// maxNeighbors (int bits), 0}.  AgentParams = one agent's record.
+struct AgentParams {
+  int k;
+  float nd_sq, obst_range_sq, radius, vmax, inv_th, inv_tho;
+};
+ORCA_HD AgentParams load_agent_params(const float4* table, const int g) {
+  const float4 r0 = ORCA_LDG(&table[2 * (size_t)g]);
+  const float4 r1 = ORCA_LDG(&table[2 * (size_t)g + 1]);
+  AgentParams q;
+  q.radius = r0.x;
+  q.vmax = r0.y;
+  q.inv_th = r0.z;
+  q.inv_tho = r0.w;
+  q.nd_sq = r1.x;
+  q.obst_range_sq = r1.y;
+  q.k = float_to_bits(r1.z);
+  return q;
+}
+
 // Where an agent's neighbor candidates come from.  TileSource: the pre-step snapshot of the
 // agent's own env in shared memory, candidates = every other agent of the env in id order.
 //
@@ -371,6 +393,9 @@ struct TileSourceT {
   ORCA_HD float2 pos(int q) const { return env_pos[q]; }
   ORCA_HD float2 vel(int q) const { return env_vel[q]; }
   ORCA_HD int local_id(int q) const { return q; }
+  // per-agent radii of the env, staged next to the snapshot (HETERO kernels only)
+  const float* env_rad = nullptr;
+  ORCA_HD float radius(int q) const { return env_rad[q]; }
 };
 using TileSource = TileSourceT<false>;
 
@@ -504,10 +529,16 @@ ORCA_HD int alan_select(const float* wrow, const int nA, const float inv_temp, c
 // uniform-grid cells), `L` is the agent's private line storage, `estep` the env's step counter
 // before this step.  Returns false when the step ends here (neighbors-only parity hook).
 // OL = obstacle-line slots of the agent's line storage (agents that need more take agent_slow_path).
-template <int K, bool KFULL, int POLICY, int OL = ORCA_MAX_OBST_LINES, class Src>
+// HETERO = the agent's ORCA parameters come from its record in `agent_params` (neighbor radii from
+// src.radius); a compile-time variant, so the uniform kernels are the code they were.  Per-agent k
+// needs the K-slot lists of KFULL = false, whose searches start from the agent's own range (no hint).
+template <int K, bool KFULL, int POLICY, int OL = ORCA_MAX_OBST_LINES, bool HETERO = false, class Src>
 ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const int estep, const Src& src,
-                         const ObstacleWorld& W, const Lines L, const unsigned warp_mask, AgentCarry& c) {
+                         const ObstacleWorld& W, const Lines L, const unsigned warp_mask, AgentCarry& c,
+                         const float4* agent_params = nullptr) {
+  static_assert(!(HETERO && KFULL), "per-agent maxNeighbors needs the KFULL = false lists");
   const float2 p = c.p, v = c.v;
+  const AgentParams ap = HETERO ? load_agent_params(agent_params, g) : AgentParams{};
 
   // ---------------- preferred velocity (policy) ----------------
   float2 gdir = v2(0.f, 0.f);
@@ -551,7 +582,7 @@ ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const in
   // uniform-grid kernel, 367 -> 357 us in config 5; in the tile kernels it measured 0 to +3.5 %, so they
   // do not compile the lookup)
   if (W.n_nodes > 0 && (!Src::kObstacleCull || obstacles_may_be_near(W, p)))
-    obstacle_neighbors(W, p, a.obst_range_sq, od, oid, &ocnt, &overflow);
+    obstacle_neighbors(W, p, HETERO ? ap.obst_range_sq : a.obst_range_sq, od, oid, &ocnt, &overflow);
 
   // Temporal coherence: where the search runs on a shrinking threshold (candidate buffer paths), it
   // starts from last step's k-th neighbor distance plus what two agents can approach each other in one
@@ -562,7 +593,10 @@ ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const in
   // from the full range.  The hint is the library's own scratch (StepArgs::nbr_hint), per agent.
   typename Src::template List<K, KFULL> nk;
   const bool hinted = KFULL && a.nbr_hint != nullptr && src.threshold_search();
-  nk.init(a.k, hinted ? fminf(a.nbr_hint[g], a.nd_sq) : a.nd_sq);
+  if (HETERO)
+    nk.init(ap.k, ap.nd_sq);
+  else
+    nk.init(a.k, hinted ? fminf(a.nbr_hint[g], a.nd_sq) : a.nd_sq);
   src.gather(nk, p, L, K + OL, warp_mask);
   if (hinted) {
     float hint = INFINITY;
@@ -608,7 +642,10 @@ ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const in
 
   // ---------------- ORCA lines ----------------
   int n_obst = 0;
-  if (ocnt > 0) n_obst = obstacle_lines<OL>(W, p, v, a.radius, a.inv_tho, od, oid, ocnt, L, &overflow);
+  if (ocnt > 0)
+    n_obst = obstacle_lines<OL>(W, p, v, HETERO ? ap.radius : a.radius, HETERO ? ap.inv_tho : a.inv_tho, od, oid, ocnt, L,
+                                &overflow);
+  const float inv_th = HETERO ? ap.inv_th : a.inv_th;
   int n = n_obst;
   unsigned collisions = 0;
   {
@@ -629,7 +666,7 @@ ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const in
         w3 >>= 8;
         bool hit;
         ORCA_DCHECK(n < K + OL);
-        const float4 ln = agent_line(p, v, src.pos(j), src.vel(j), cr, a.inv_th, a.inv_dt, &hit);
+        const float4 ln = agent_line(p, v, src.pos(j), src.vel(j), HETERO ? ap.radius + src.radius(j) : cr, inv_th, a.inv_dt, &hit);
         L.base[n * L.stride] = ln;
         ++n;
         collisions += hit ? 1u : 0u;
@@ -657,7 +694,7 @@ ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const in
           vn = src.vel(jn);
         }
         bool hit;
-        const float4 ln = agent_line(p, v, pj, vj, cr, a.inv_th, a.inv_dt, &hit);
+        const float4 ln = agent_line(p, v, pj, vj, HETERO ? ap.radius + src.radius(j) : cr, inv_th, a.inv_dt, &hit);
         L.base[n * L.stride] = ln;
         ++n;
         collisions += hit ? 1u : 0u;
@@ -674,7 +711,7 @@ ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const in
         const int j = nk.id[s];
         if (j >= 0) {
           bool hit;
-          const float4 ln = agent_line(p, v, src.pos(j), src.vel(j), cr, a.inv_th, a.inv_dt, &hit);
+          const float4 ln = agent_line(p, v, src.pos(j), src.vel(j), HETERO ? ap.radius + src.radius(j) : cr, inv_th, a.inv_dt, &hit);
           L.base[n * L.stride] = ln;
           ++n;
           collisions += hit ? 1u : 0u;
@@ -689,7 +726,7 @@ ORCA_HD bool agent_front(const StepArgs& a, const int env, const int g, const in
   c.overflow = overflow;
 
   // ---------------- LP2 ----------------
-  c.fail = lp2(warp_mask, true, L, n, a.vmax, pref, false, c.nv);
+  c.fail = lp2(warp_mask, true, L, n, HETERO ? ap.vmax : a.vmax, pref, false, c.nv);
   return true;
 }
 
@@ -727,7 +764,21 @@ ORCA_HD SlowParams slow_params(const StepArgs& a) {
   q.obst_range_sq = a.obst_range_sq;
   return q;
 }
-template <int K, bool KFULL, class Src>
+// ... of agent g from its record (HETERO kernels)
+ORCA_HD SlowParams slow_params(const StepArgs& a, const float4* agent_params, const int g) {
+  const AgentParams ap = load_agent_params(agent_params, g);
+  SlowParams q;
+  q.k = ap.k;
+  q.nd_sq = ap.nd_sq;
+  q.inv_th = ap.inv_th;
+  q.inv_tho = ap.inv_tho;
+  q.inv_dt = a.inv_dt;
+  q.radius = ap.radius;
+  q.vmax = ap.vmax;
+  q.obst_range_sq = ap.obst_range_sq;
+  return q;
+}
+template <int K, bool KFULL, class Src, bool HETERO = false>
 ORCA_HD_NOINLINE SlowResult agent_slow_path(const SlowParams a, const Src src, const ObstacleWorld W, const Lines scratch,
                                             const int scratch_slots, const unsigned mask, const float2 p, const float2 v,
                                             const float2 pref) {
@@ -752,7 +803,7 @@ ORCA_HD_NOINLINE SlowResult agent_slow_path(const SlowParams a, const Src src, c
     const int j = nk.id[s];
     if (j >= 0) {
       bool hit;
-      buf[n++] = agent_line(p, v, src.pos(j), src.vel(j), cr, a.inv_th, a.inv_dt, &hit);
+      buf[n++] = agent_line(p, v, src.pos(j), src.vel(j), HETERO ? a.radius + src.radius(j) : cr, a.inv_th, a.inv_dt, &hit);
       collisions += hit ? 1u : 0u;
     }
   }
@@ -854,20 +905,21 @@ ORCA_HD void agent_back(const StepArgs& a, const int env, const int la, const in
 }
 
 // Front + LP3 + back for one agent, no work redistribution (host emulation; reference order).
-template <int K, bool KFULL, int POLICY, class Src>
+template <int K, bool KFULL, int POLICY, bool HETERO = false, class Src>
 ORCA_HD void agent_step_body(const StepArgs& a, const int env, const int la, const int g, float2 p, float2 v,
-                             const int estep, const Src& src, const Lines L, const unsigned warp_mask) {
+                             const int estep, const Src& src, const Lines L, const unsigned warp_mask,
+                             const float4* agent_params = nullptr) {
   AgentCarry c;
   c.p = p;
   c.v = v;
   c.aim = (POLICY == POLICY_EXTERNAL) ? a.pref[g] : a.goal[g];
   const ObstacleWorld W = Src::kObstacleCull ? global_world_with_cull(a, env) : global_world(a, env);
-  if (!agent_front<K, KFULL, POLICY>(a, env, g, estep, src, W, L, warp_mask, c)) return;
+  if (!agent_front<K, KFULL, POLICY, ORCA_MAX_OBST_LINES, HETERO>(a, env, g, estep, src, W, L, warp_mask, c, agent_params)) return;
   if (c.overflow)
-    apply_slow_result(agent_slow_path<K, KFULL>(slow_params(a), src, global_world(a, env), L, K + ORCA_MAX_OBST_LINES, warp_mask,
-                                                c.p, c.v, c.pref), c);
+    apply_slow_result(agent_slow_path<K, KFULL, Src, HETERO>(HETERO ? slow_params(a, agent_params, g) : slow_params(a), src, global_world(a, env), L,
+                                                             K + ORCA_MAX_OBST_LINES, warp_mask, c.p, c.v, c.pref), c);
   else
-    lp3(warp_mask, c.fail < c.n, L, c.n, c.n_obst, c.fail, a.vmax, c.nv);
+    lp3(warp_mask, c.fail < c.n, L, c.n, c.n_obst, c.fail, HETERO ? load_agent_params(agent_params, g).vmax : a.vmax, c.nv);
   agent_back<POLICY>(a, env, la, g, estep, c);
 }
 
@@ -885,8 +937,11 @@ ORCA_HD void agent_step_body(const StepArgs& a, const int env, const int la, con
 #define ORCA_LP3_SMEM_POOL 0
 #endif
 // dynamic shared memory of the step kernels: [pos|vel tile (tile path only)] + lines + LP3 queue
-inline size_t step_smem_bytes(int K, int tpb, bool tile, int world_slots = 0, int obst_lines = ORCA_MAX_OBST_LINES) {
+inline size_t step_smem_bytes(int K, int tpb, bool tile, int world_slots = 0, int obst_lines = ORCA_MAX_OBST_LINES,
+                              bool hetero = false) {
   size_t b = (size_t)world_slots * 64 + 16;  // staged obstacle tables: 4 x 16 B per vertex slot
+  // HETERO kernels: each thread's agent's maxSpeed (for block_lp3) and, in the tile, the agents' radii
+  if (hetero) b += (size_t)tpb * (tile ? 8 : 4);
   // per thread: tile (pos, vel) + lines + LP3 queue (nv 8, meta 4, queue entry 1); per block: 8 warp counters
   b += (size_t)tpb * ((tile ? 16 : 0) + (size_t)(K + obst_lines) * 16 + 8 + 4 + 1) + 8 * 4;
 #if ORCA_LP3_SMEM_POOL
@@ -908,10 +963,12 @@ inline size_t step_smem_bytes(int K, int tpb, bool tile, int world_slots = 0, in
 #ifndef ORCA_LP3_SMEM_POOL
 #define ORCA_LP3_SMEM_POOL 0
 #endif
-template <int K>
+// HETERO: a solver works on another thread's agent and takes that OWNER's maxSpeed from s_vmax
+// (one entry per thread, written before the call); otherwise every agent has `vmax`.
+template <int K, bool HETERO = false>
 __device__ __forceinline__ void block_lp3(float4* s_lines, float4* s_pool, int* s_meta, float2* s_nv,
                                           unsigned char* s_queue, int* s_warp_cnt, const bool need, const AgentCarry& c, const float vmax,
-                                          const bool area_was_borrowed = false) {
+                                          const bool area_was_borrowed = false, const float* s_vmax = nullptr) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
   // the queue area doubled as the in-block neighbor grid during the front half: nobody may
   // overwrite it while another warp still searches its neighbors
@@ -922,7 +979,7 @@ __device__ __forceinline__ void block_lp3(float4* s_lines, float4* s_pool, int* 
     L.base = s_lines + tid;
     L.stride = blockDim.x;
     float2 nv = c.nv;
-    lp3(0xffffffffu, need, L, c.n, c.n_obst, c.fail, vmax, nv);
+    lp3(0xffffffffu, need, L, c.n, c.n_obst, c.fail, HETERO ? s_vmax[tid] : vmax, nv);
     s_nv[tid] = nv;
     __syncwarp();
     return;
@@ -966,7 +1023,7 @@ __device__ __forceinline__ void block_lp3(float4* s_lines, float4* s_pool, int* 
       P.base = s_pool + tid;
       P.stride = pool;
       float2 nv = s_nv[owner];
-      lp3_stored(0xffffffffu, mine, L, meta & 0xff, (meta >> 8) & 0xff, (meta >> 16) & 0xff, vmax, P, nv);
+      lp3_stored(0xffffffffu, mine, L, meta & 0xff, (meta >> 8) & 0xff, (meta >> 16) & 0xff, HETERO ? s_vmax[owner] : vmax, P, nv);
       if (mine) s_nv[owner] = nv;
     }
   }
@@ -1001,9 +1058,9 @@ __device__ __forceinline__ void block_lp3(float4* s_lines, float4* s_pool, int* 
       Lines P;
       P.base = s_lines + (mine ? (int)s_queue[blockDim.x - 1 - tid] : tid);
       P.stride = blockDim.x;
-      lp3_stored(0xffffffffu, mine, L, meta & 0xff, (meta >> 8) & 0xff, (meta >> 16) & 0xff, vmax, P, nv);
+      lp3_stored(0xffffffffu, mine, L, meta & 0xff, (meta >> 8) & 0xff, (meta >> 16) & 0xff, HETERO ? s_vmax[owner] : vmax, P, nv);
     } else {
-      lp3(0xffffffffu, mine, L, meta & 0xff, (meta >> 8) & 0xff, (meta >> 16) & 0xff, vmax, nv);
+      lp3(0xffffffffu, mine, L, meta & 0xff, (meta >> 8) & 0xff, (meta >> 16) & 0xff, HETERO ? s_vmax[owner] : vmax, nv);
     }
     if (mine) s_nv[owner] = nv;
   }
@@ -1088,8 +1145,10 @@ __device__ __forceinline__ void build_tile_grid(const StepArgs& a, void* area, c
 // shared memory per thread, which lets FOUR 256-thread blocks share an SM (64 registers) instead of three.
 // Measured (config 2, 214 us at 3 blocks): 2 blocks 272 us, 1 block 480 us -- resident warps are what hides
 // the dependent-instruction latency of the LP chains.
-template <int K, bool KFULL, int POLICY, int OL = ORCA_MAX_OBST_LINES>
-__global__ void __launch_bounds__(ORCA_STEP_MAX_THREADS, ((OL <= 2 || K <= 5) ? 4 : ORCA_STEP_MIN_BLOCKS)) step_small_kernel(const StepArgs a) {
+// HETERO: per-agent parameters (agent_front); the radii of the block's agents are staged after the
+// obstacle tables, next to one maxSpeed per thread for block_lp3.
+template <int K, bool KFULL, int POLICY, int OL = ORCA_MAX_OBST_LINES, bool HETERO = false>
+__global__ void __launch_bounds__(ORCA_STEP_MAX_THREADS, ((OL <= 2 || K <= 5) ? 4 : ORCA_STEP_MIN_BLOCKS)) step_small_kernel(const StepArgs a, const float4* __restrict__ agent_params) {
   extern __shared__ float4 smem4[];
   const int tpb = blockDim.x;
   // [pos | vel] tile: 2 * tpb float2 = tpb float4 ; lines: (K + OL) * tpb float4 ;
@@ -1104,6 +1163,8 @@ __global__ void __launch_bounds__(ORCA_STEP_MAX_THREADS, ((OL <= 2 || K <= 5) ? 
   unsigned char* s_queue = reinterpret_cast<unsigned char*>(s_warp_cnt + 8);
   // staged obstacle tables (16-byte aligned, after the queue): vert_pd | vert_link | bsp | bsp_seg
   float4* s_world = reinterpret_cast<float4*>((reinterpret_cast<uintptr_t>(s_queue + tpb) + 15) & ~(uintptr_t)15);
+  float* s_rad = reinterpret_cast<float*>(s_world + 4 * a.world_slots);
+  float* s_vmax = s_rad + tpb;
 
   const int tid = threadIdx.x;
   const int N = a.N;
@@ -1130,6 +1191,7 @@ __global__ void __launch_bounds__(ORCA_STEP_MAX_THREADS, ((OL <= 2 || K <= 5) ? 
     c.v = a.vel[g];
     s_pos[tid] = c.p;
     s_vel[tid] = c.v;
+    if (HETERO) s_rad[tid] = ORCA_LDG(&agent_params[2 * (size_t)g]).x;
     if (a.env_step != nullptr) estep = a.env_step[env];
     // read before the first barrier: nobody of this env (= this block) has counted an arrival of this step yet
     if (a.env_done_cnt != nullptr) env_live = a.env_done_cnt[env] < N;
@@ -1191,11 +1253,14 @@ __global__ void __launch_bounds__(ORCA_STEP_MAX_THREADS, ((OL <= 2 || K <= 5) ? 
     src.env_vel = s_vel + le * N;
     src.n = N;
     src.self = la;
-    src.full_range_sq = a.nd_sq;
-    alive = agent_front<K, KFULL, POLICY, OL>(a, env, g, estep, src, W, L, warp_mask, c);
+    src.full_range_sq = HETERO ? ORCA_LDG(&agent_params[2 * (size_t)g + 1]).x : a.nd_sq;
+    if (HETERO) src.env_rad = s_rad + le * N;
+    alive = agent_front<K, KFULL, POLICY, OL, HETERO>(a, env, g, estep, src, W, L, warp_mask, c, agent_params);
+    if (HETERO) s_vmax[tid] = ORCA_LDG(&agent_params[2 * (size_t)g]).y;
   }
   if (a.neighbors_only) return;  // uniform over the grid
-  block_lp3<K>(s_lines, s_pool, s_meta, s_nv, s_queue, s_warp_cnt, alive && !c.overflow && c.fail < c.n, c, a.vmax, tile_grid);
+  block_lp3<K, HETERO>(s_lines, s_pool, s_meta, s_nv, s_queue, s_warp_cnt, alive && !c.overflow && c.fail < c.n, c, a.vmax, tile_grid,
+                       s_vmax);
   const unsigned slow_mask = __ballot_sync(0xffffffffu, alive && c.overflow);
   if (!alive) return;
   c.nv = s_nv[tid];
@@ -1211,7 +1276,9 @@ __global__ void __launch_bounds__(ORCA_STEP_MAX_THREADS, ((OL <= 2 || K <= 5) ? 
     scan.env_vel = s_vel + le * N;
     scan.n = N;
     scan.self = la;
-    apply_slow_result(agent_slow_path<K, KFULL>(slow_params(a), scan, global_world(a, env), L, K + OL, slow_mask, c.p, c.v, c.pref), c);
+    if (HETERO) scan.env_rad = s_rad + le * N;
+    apply_slow_result(agent_slow_path<K, KFULL, Source, HETERO>(HETERO ? slow_params(a, agent_params, g) : slow_params(a), scan, global_world(a, env), L,
+                                                                K + OL, slow_mask, c.p, c.v, c.pref), c);
   }
   agent_back<POLICY>(a, env, la, g, estep, c, env_live);
 }

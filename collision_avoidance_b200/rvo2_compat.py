@@ -8,8 +8,12 @@ run unmodified against the CUDA path (tests/test_gpu_compat.py replays the recor
 compatibility shim, not the fast path: every ``doStep`` is one kernel launch for one world plus
 host<->device mirrors; throughput comes from ``BatchedRVOSimulator`` / ``envs`` / ``alan``.
 
-Restrictions (checked, never silent): all agents of a simulator share their parameters (the
-reference always passes the same ones), ``maxNeighbors <= 16``.
+Agents may have parameters of their own, as in RVO2: ``addAgent`` takes all six per agent, and
+``getAgent``/``setAgent`` ``NeighborDist``, ``MaxNeighbors``, ``TimeHorizon``, ``TimeHorizonObst``,
+``Radius`` and ``MaxSpeed`` read and change them between steps.  A world whose agents all share one
+set runs the uniform kernels; a mixed one uploads its per-agent table before the next ``doStep``.
+
+Restrictions (checked, never silent): ``maxNeighbors <= 16``.
 """
 from __future__ import annotations
 
@@ -30,7 +34,10 @@ class PyRVOSimulator:
                           float(radius), float(maxSpeed))
         self._default_velocity = (float(velocity[0]), float(velocity[1]))
         self._device = device
-        self._agent_params: Optional[Tuple] = None
+        self._params: List[Tuple] = []     # per agent: (neighborDist, maxNeighbors, timeHorizon, timeHorizonObst, radius, maxSpeed)
+        self._params_dirty = True          # the table on the device (if any) is older than self._params
+        self._sim_params: Optional[Tuple] = None  # the OrcaParams the current simulator was built with
+        self._table_set = False
         self._pos: List[Tuple[float, float]] = []
         self._vel: List[Tuple[float, float]] = []
         self._pref: List[Tuple[float, float]] = []
@@ -54,11 +61,8 @@ class PyRVOSimulator:
             params = (float(neighborDist), int(maxNeighbors), float(timeHorizon), float(timeHorizonObst),
                       float(radius), float(maxSpeed))
             vel = (float(velocity[0]), float(velocity[1]))
-        if self._agent_params is None:
-            self._agent_params = params
-        elif params != self._agent_params:
-            raise NotImplementedError("all agents of a simulator must share their parameters "
-                                      f"(first agent: {self._agent_params}, this one: {params})")
+        self._params.append(tuple(self._f32(x) if i != 1 else x for i, x in enumerate(params)))
+        self._params_dirty = True
         self._pos.append((float(np.float32(pos[0])), float(np.float32(pos[1]))))
         self._vel.append((float(np.float32(vel[0])), float(np.float32(vel[1]))))
         self._pref.append((0.0, 0.0))
@@ -83,16 +87,44 @@ class PyRVOSimulator:
             self._sim.set_obstacles([p for p in self._polygons])
 
     # ------------------------------------------------------------------ device plumbing
+    @staticmethod
+    def _f32(x) -> float:
+        return float(np.float32(x))
+
+    def _handle_params(self):
+        """(OrcaParams of the simulator, whether the agents need a per-agent table).  Shared
+        parameters are the simulator's own; otherwise the first agent's, with the largest maxNeighbors."""
+        first = self._params[0]
+        if all(p == first for p in self._params):
+            return first, False
+        return (first[0], max(p[1] for p in self._params)) + first[2:], True
+
     def _ensure_sim(self) -> BatchedRVOSimulator:
+        if not self._pos:
+            raise RuntimeError("no agents in the simulation")
+        hp, hetero = self._handle_params()
+        if self._sim is not None and hp != self._sim_params:
+            self._sim = None  # another maxNeighbors bound (or another shared set): rebuild
         if self._sim is None:
-            if not self._pos:
-                raise RuntimeError("no agents in the simulation")
-            nd, k, th, tho, r, vmax = self._agent_params
+            nd, k, th, tho, r, vmax = hp
             self._sim = BatchedRVOSimulator(1, len(self._pos), self._time_step, nd, k, th, tho, r, vmax,
                                             device=self._device)
+            self._sim_params = hp
+            self._table_set = False
+            self._params_dirty = True
             if self._processed:
                 self._sim.set_obstacles([p for p in self._polygons])
             self._dirty = True
+        if self._params_dirty:
+            if hetero:
+                cols = list(zip(*self._params))
+                self._sim.set_agent_params(
+                    *(np.asarray(c, np.int32 if j == 1 else np.float32).reshape(1, -1) for j, c in enumerate(cols)))
+                self._table_set = True
+            elif self._table_set:
+                self._sim.set_agent_params()
+                self._table_set = False
+            self._params_dirty = False
         return self._sim
 
     def _vertices(self):
@@ -182,6 +214,49 @@ class PyRVOSimulator:
     def getObstacleVertex(self, v):
         p = self._vertices()[0][v]
         return (float(p[0]), float(p[1]))
+
+    # per-agent parameters (RVO2's getAgent* / setAgent*); a change takes effect at the next doStep
+    def _set_param(self, i, j, value):
+        p = list(self._params[i])
+        p[j] = int(value) if j == 1 else self._f32(value)
+        self._params[i] = tuple(p)
+        self._params_dirty = True
+
+    def getAgentNeighborDist(self, i):
+        return self._params[i][0]
+
+    def getAgentMaxNeighbors(self, i):
+        return self._params[i][1]
+
+    def getAgentTimeHorizon(self, i):
+        return self._params[i][2]
+
+    def getAgentTimeHorizonObst(self, i):
+        return self._params[i][3]
+
+    def getAgentRadius(self, i):
+        return self._params[i][4]
+
+    def getAgentMaxSpeed(self, i):
+        return self._params[i][5]
+
+    def setAgentNeighborDist(self, i, neighborDist):
+        self._set_param(i, 0, neighborDist)
+
+    def setAgentMaxNeighbors(self, i, maxNeighbors):
+        self._set_param(i, 1, maxNeighbors)
+
+    def setAgentTimeHorizon(self, i, timeHorizon):
+        self._set_param(i, 2, timeHorizon)
+
+    def setAgentTimeHorizonObst(self, i, timeHorizonObst):
+        self._set_param(i, 3, timeHorizonObst)
+
+    def setAgentRadius(self, i, radius):
+        self._set_param(i, 4, radius)
+
+    def setAgentMaxSpeed(self, i, maxSpeed):
+        self._set_param(i, 5, maxSpeed)
 
     def getNumAgents(self):
         return len(self._pos)

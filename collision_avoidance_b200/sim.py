@@ -32,8 +32,11 @@ class BatchedRVOSimulator:
     """Batch of ORCA worlds on one GPU.
 
     Constructor arguments are those of ``rvo2.PyRVOSimulator`` (ALAN_true.py:22-28) plus the
-    batch shape.  All agents share the parameters, as they do everywhere in the reference
-    (collision_avoidence_env.py:126-133, ALAN_true.py:461-468).
+    batch shape.  They are every agent's parameters, as everywhere in the reference
+    (collision_avoidence_env.py:126-133, ALAN_true.py:461-468), until ``set_agent_params`` gives
+    agents their own neighborDist, maxNeighbors, timeHorizon, timeHorizonObst, radius and maxSpeed
+    (RVO2's per-agent addAgent arguments).  The time step, the done test's 2 * radius and
+    ``observe`` stay those of the constructor.
     """
 
     def __init__(self, num_envs: int, agents_per_env: int, timeStep: float, neighborDist: float, maxNeighbors: int,
@@ -93,6 +96,38 @@ class BatchedRVOSimulator:
         if t.dtype != dtype or tuple(t.shape) != tuple(shape) or not t.is_contiguous() or not t.is_cuda:
             raise ValueError(f"{name} must be a contiguous CUDA {dtype} tensor of shape {tuple(shape)}, "
                              f"got {t.dtype} {tuple(t.shape)}")
+
+    # ------------------------------------------------------------------ per-agent parameters
+    _AGENT_PARAMS = (("neighbor_dist", np.float32), ("max_neighbors", np.int32), ("time_horizon", np.float32),
+                     ("time_horizon_obst", np.float32), ("radius", np.float32), ("max_speed", np.float32))
+
+    def set_agent_params(self, neighbor_dist=None, max_neighbors=None, time_horizon=None, time_horizon_obst=None,
+                         radius=None, max_speed=None):
+        """Per-agent ORCA parameters (RVO2's addAgent / setAgent{NeighborDist,MaxNeighbors,TimeHorizon,
+        TimeHorizonObst,Radius,MaxSpeed}).  Each argument is an ``[E, N]`` array or tensor (CPU or CUDA),
+        copied to the host once; ``None`` = the constructor's value for every agent.  All ``None``
+        returns to uniform parameters.  ``max_neighbors`` must lie in [0, maxNeighbors of the
+        constructor]; time horizons must be > 0, the others >= 0, all finite (``ValueError``).
+        Synchronises with the device, like ``set_obstacles``."""
+        given = dict(neighbor_dist=neighbor_dist, max_neighbors=max_neighbors, time_horizon=time_horizon,
+                     time_horizon_obst=time_horizon_obst, radius=radius, max_speed=max_speed)
+        shape = (self.num_envs, self.agents_per_env)
+        arrays = {}
+        for name, dtype in self._AGENT_PARAMS:
+            v = given[name]
+            if v is None:
+                arrays[name] = None
+                continue
+            if isinstance(v, torch.Tensor):
+                v = v.detach().cpu().numpy()
+            v = np.asarray(v)
+            if tuple(v.shape) != shape:
+                raise ValueError(f"{name} must have shape {shape}, got {tuple(v.shape)}")
+            if dtype is np.int32 and not np.issubdtype(v.dtype, np.integer):
+                raise ValueError(f"{name} must be integral, got {v.dtype}")
+            arrays[name] = np.ascontiguousarray(v, dtype)
+        ptr = lambda a: None if a is None else a.ctypes.data
+        _lib.check(self._L.orca_set_agent_params(self._h, *(ptr(arrays[n]) for n, _ in self._AGENT_PARAMS)))
 
     # ------------------------------------------------------------------ obstacles
     def set_obstacles(self, polygons: Sequence, per_env: bool = False):

@@ -40,7 +40,7 @@ typedef enum OrcaStatus {
  * rvo2.PyRVOSimulator(timeStep, neighborDist, maxNeighbors, timeHorizon,
  * timeHorizonObst, radius, maxSpeed)  -- ALAN_true.py:22-28, collision_avoidence_env.py:62-68,
  * and of addAgent(...) -- collision_avoidence_env.py:126-133, ALAN_true.py:461-468.
- * All agents of a handle share them (the reference never varies them per agent). */
+ * They are every agent's parameters unless orca_set_agent_params gives agents their own. */
 typedef struct OrcaParams {
   float time_step;
   float neighbor_dist;
@@ -159,6 +159,20 @@ const char* orca_last_error(void);
 int orca_create(const OrcaParams* params, int device, int num_envs, int agents_per_env, OrcaSim** out);
 int orca_destroy(OrcaSim* sim);
 int orca_get_params(const OrcaSim* sim, OrcaParams* out, int* num_envs, int* agents_per_env);
+
+/* Per-agent ORCA parameters: RVO2's addAgent(pos, neighborDist, maxNeighbors, timeHorizon,
+ * timeHorizonObst, radius, maxSpeed, velocity) and its setAgent{NeighborDist,MaxNeighbors,
+ * TimeHorizon,TimeHorizonObst,Radius,MaxSpeed}.  HOST arrays of E*N entries, env-major.
+ * A NULL array means every agent takes the handle's OrcaParams value.  All six NULL returns the
+ * handle to uniform parameters.  The values are copied; the call synchronises (a setup call,
+ * like orca_set_obstacles).  ORCA_ERR_INVALID unless every value is finite, time_horizon and
+ * time_horizon_obst > 0, neighbor_dist, radius, max_speed >= 0 and 0 <= max_neighbors <=
+ * OrcaParams.max_neighbors (which stays the row width of the neighbor-list outputs).
+ * Handle-wide whatever the table holds: the time step, the 2 * radius of the done test and
+ * orca_observe (its neighbor octagons use OrcaParams.radius, its rays OrcaParams.neighbor_dist). */
+int orca_set_agent_params(OrcaSim* sim, const float* neighbor_dist, const int32_t* max_neighbors,
+                          const float* time_horizon, const float* time_horizon_obst,
+                          const float* radius, const float* max_speed);
 
 /* ---- obstacles -------------------------------------------------------------------
  * Replaces addObstacle(...) x P + processObstacles() (collision_avoidence_env.py:118-123,145;
