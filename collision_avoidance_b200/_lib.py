@@ -35,6 +35,7 @@ MAX_ACTIONS = 16
 EXPORTED_SYMBOLS = (
     "orca_abi_version", "orca_last_error", "orca_create", "orca_destroy", "orca_get_params", "orca_set_agent_params",
     "orca_set_obstacles", "orca_obstacle_vertex_count", "orca_get_obstacle_vertices",
+    "orca_query_visibility", "orca_set_roadmap", "orca_get_roadmap", "orca_roadmap_pref_velocity",
     "orca_step", "orca_env_step", "orca_env_step_many", "orca_neighbors", "orca_observe", "orca_step_host", "orca_step_host_ex", "orca_policy_mlp", "orca_policy_mlp_fp32", "orca_launch_count",
 )
 
@@ -131,6 +132,10 @@ def load() -> ctypes.CDLL:
     L.orca_set_obstacles.argtypes = [hp, _vp, _vp, i, _vp]
     L.orca_obstacle_vertex_count.argtypes = [hp, i]
     L.orca_get_obstacle_vertices.argtypes = [hp, i, _vp, _vp, _vp, _vp]
+    L.orca_query_visibility.argtypes = [hp, _vp, _vp, _vp, f, i, _vp, _vp]
+    L.orca_set_roadmap.argtypes = [hp, _vp, i, i, i, f]
+    L.orca_get_roadmap.argtypes = [hp, i, _vp, _vp]
+    L.orca_roadmap_pref_velocity.argtypes = [hp, _vp, _vp, _vp, _vp, _vp]
     L.orca_step.argtypes = [hp, _vp, _vp, _vp, _vp]
     L.orca_env_step.argtypes = [hp, ctypes.POINTER(OrcaEnvStepArgs), _vp]
     L.orca_env_step_many.argtypes = [hp, ctypes.POINTER(OrcaEnvStepArgs), i, _vp]

@@ -24,6 +24,7 @@
 #include "orca_obs.cuh"
 #include "orca_policy.cuh"
 #include "orca_policy_tc.cuh"
+#include "orca_roadmap.cuh"
 #include "orca_step_small.cuh"
 
 namespace {
@@ -116,6 +117,16 @@ struct OrcaSim {
   float4* d_agent_params = nullptr;
   float max_nd = 0.f, max_orange = 0.f;
   float cull_range = 0.f;  // obstacle range the obstacle-free maps were built for
+  // roadmap (orca_set_roadmap): the caller's vertices are kept on the host so that orca_set_obstacles
+  // can rebuild the edges and distances; rm_R == 0 means no roadmap
+  std::vector<float> rm_host_xy;  // [1 or E][R][2]
+  int rm_R = 0, rm_G = 0;
+  bool rm_per_env = false;
+  float rm_radius = 0.f;
+  int rm_tables = 0;                // table sets on the device: E when the obstacles or the roadmap are per env, else 1
+  float2* d_rm_xy = nullptr;
+  uint32_t* d_rm_adj = nullptr;
+  float* d_rm_dist = nullptr;
   // uniform-grid scratch (large worlds)
   orca::GridScratch grid;
   int64_t launches = 0;
@@ -338,6 +349,69 @@ int build_cull_maps(OrcaSim* s) {
   return ORCA_OK;
 }
 
+orca::BspTables bsp_tables(const OrcaSim* s) {
+  orca::BspTables T;
+  T.bsp = s->d_bsp;
+  T.bsp_seg = s->d_bsp_seg;
+  T.env_nodes = s->per_env ? s->d_env_nodes : nullptr;
+  T.shared_nodes = s->shared_nodes;
+  T.vert_stride = s->per_env ? s->vert_stride : 0;
+  return T;
+}
+
+orca::RoadmapArgs roadmap_args(const OrcaSim* s) {
+  orca::RoadmapArgs a;
+  a.bsp = bsp_tables(s);
+  a.W = s->rm_tables;
+  a.R = s->rm_R;
+  a.G = s->rm_G;
+  a.words = (s->rm_R + 31) / 32;
+  a.xy_per_table = s->rm_per_env ? 1 : 0;
+  a.obst_per_table = (s->per_env && s->vert_stride > 0) ? 1 : 0;
+  a.radius = s->rm_radius;
+  a.xy = s->d_rm_xy;
+  a.adj = s->d_rm_adj;
+  a.dist = s->d_rm_dist;
+  return a;
+}
+
+void free_roadmap_tables(OrcaSim* s) {
+  cudaFree(s->d_rm_xy);
+  cudaFree(s->d_rm_adj);
+  cudaFree(s->d_rm_dist);
+  s->d_rm_xy = nullptr;
+  s->d_rm_adj = nullptr;
+  s->d_rm_dist = nullptr;
+  s->rm_tables = 0;
+}
+
+// Edges and goal distances of the kept roadmap over the current obstacle worlds (Roadmap.cpp
+// buildRoadmap), computed on the device; synchronises.
+int build_roadmap(OrcaSim* s) {
+  free_roadmap_tables(s);
+  if (s->rm_R == 0) return ORCA_OK;
+  const int R = s->rm_R, G = s->rm_G, words = (R + 31) / 32;
+  const int W = (s->rm_per_env || s->per_env) ? s->E : 1;
+  const size_t xy_rows = s->rm_per_env ? (size_t)s->E : 1;
+  CUDA_TRY(cudaMalloc(&s->d_rm_xy, xy_rows * R * sizeof(float2)));
+  CUDA_TRY(cudaMalloc(&s->d_rm_adj, (size_t)W * R * words * sizeof(uint32_t)));
+  CUDA_TRY(cudaMalloc(&s->d_rm_dist, (size_t)W * G * R * sizeof(float)));
+  CUDA_TRY(cudaMemcpy(s->d_rm_xy, s->rm_host_xy.data(), xy_rows * R * sizeof(float2), cudaMemcpyHostToDevice));
+  s->rm_tables = W;
+  const orca::RoadmapArgs a = roadmap_args(s);
+  const long long threads = (long long)W * R * words * 32;
+  orca::roadmap_edges_kernel<<<(unsigned)((threads + 255) / 256), 256>>>(a);
+  CUDA_TRY(cudaGetLastError());
+  // one thread per vertex (R <= 512); shared memory: vertices, adjacency, distances
+  const int tpb = std::max(32, (R + 31) / 32 * 32);
+  const size_t smem = (size_t)R * sizeof(float2) + (size_t)R * words * sizeof(uint32_t) + (size_t)R * sizeof(float);
+  orca::roadmap_dist_kernel<<<(unsigned)((long long)W * G), tpb, smem>>>(a);
+  CUDA_TRY(cudaGetLastError());
+  s->launches += 2;
+  CUDA_TRY(cudaDeviceSynchronize());
+  return ORCA_OK;
+}
+
 int ensure_host_staging(OrcaSim* s) {
   if (s->d_pos != nullptr) return ORCA_OK;
   const size_t bytes = (size_t)s->E * s->N * sizeof(float2);
@@ -399,6 +473,7 @@ int orca_destroy(OrcaSim* s) {
   if (s == nullptr) return ORCA_OK;
   DeviceGuard guard(s->device);
   free_obstacles(s);
+  free_roadmap_tables(s);
   cudaFree(s->d_pos);
   cudaFree(s->d_vel);
   cudaFree(s->d_aux);
@@ -455,7 +530,7 @@ int orca_set_obstacles(OrcaSim* s, const float* xy, const int32_t* poly_sizes, i
   if (poly != num_polys) return fail(ORCA_ERR_INVALID, "polys_per_env does not cover all polygons");
   int stride = 0;
   for (const auto& T : s->worlds) stride = T.num_vertices() > stride ? T.num_vertices() : stride;
-  if (stride == 0) return ORCA_OK;  // no obstacles at all
+  if (stride == 0) return build_roadmap(s);  // no obstacles at all
   std::vector<float4> pd((size_t)n_worlds * stride), seg((size_t)n_worlds * stride);
   std::vector<int4> link((size_t)n_worlds * stride), bsp((size_t)n_worlds * stride);
   std::vector<int> nodes((size_t)n_worlds);
@@ -495,7 +570,9 @@ int orca_set_obstacles(OrcaSim* s, const float* xy, const int32_t* poly_sizes, i
   }
   s->shared_nodes = s->per_env ? 0 : nodes[0];
   s->vert_stride = stride;
-  return build_cull_maps(s);
+  const int rc = build_cull_maps(s);
+  if (rc != ORCA_OK) return rc;
+  return build_roadmap(s);  // the roadmap's edges and distances depend on the obstacles
 }
 
 int orca_set_agent_params(OrcaSim* s, const float* neighbor_dist, const int32_t* max_neighbors, const float* time_horizon,
@@ -573,6 +650,92 @@ int orca_get_obstacle_vertices(const OrcaSim* s, int env, float* xy_out, int32_t
     if (prev_out) prev_out[v] = T.prev[(size_t)v];
     if (convex_out) convex_out[v] = T.convex[(size_t)v];
   }
+  return ORCA_OK;
+}
+
+int orca_query_visibility(OrcaSim* s, const float* q1_dev, const float* q2_dev, const float* radius_dev, float radius,
+                          int queries_per_env, uint8_t* visible_dev, void* stream) {
+  if (s == nullptr) return fail(ORCA_ERR_INVALID, "null handle");
+  if (queries_per_env < 0) return fail(ORCA_ERR_INVALID, "queries_per_env must be >= 0");
+  if (queries_per_env == 0) return ORCA_OK;
+  if (q1_dev == nullptr || q2_dev == nullptr || visible_dev == nullptr)
+    return fail(ORCA_ERR_INVALID, "orca_query_visibility: null pointer argument");
+  if (radius_dev == nullptr && !(std::isfinite(radius) && radius >= 0.f))
+    return fail(ORCA_ERR_INVALID, "radius must be finite and >= 0");
+  const long long total = (long long)s->E * queries_per_env;
+  if (total >= (1ll << 38)) return fail(ORCA_ERR_UNSUPPORTED, "E * queries_per_env must be below 2^38");
+  DeviceGuard guard(s->device);
+  orca::visibility_kernel<<<(unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      bsp_tables(s), s->E, queries_per_env, reinterpret_cast<const float2*>(q1_dev), reinterpret_cast<const float2*>(q2_dev),
+      radius_dev, radius, visible_dev);
+  CUDA_TRY(cudaGetLastError());
+  s->launches += 1;
+  return ORCA_OK;
+}
+
+int orca_set_roadmap(OrcaSim* s, const float* xy, int num_vertices, int num_goals, int per_env, float radius) {
+  if (s == nullptr) return fail(ORCA_ERR_INVALID, "null handle");
+  if (num_vertices < 0) return fail(ORCA_ERR_INVALID, "num_vertices must be >= 0");
+  std::vector<float> host;
+  if (num_vertices > 0) {
+    if (num_vertices > orca::kRoadmapMaxVertices)
+      return fail(ORCA_ERR_UNSUPPORTED, "a roadmap has at most %d vertices (got %d)", orca::kRoadmapMaxVertices, num_vertices);
+    if (num_goals < 1 || num_goals > num_vertices)
+      return fail(ORCA_ERR_UNSUPPORTED, "num_goals must be in [1, num_vertices] (got %d of %d)", num_goals, num_vertices);
+    if (xy == nullptr) return fail(ORCA_ERR_INVALID, "null vertex array");
+    if (!(std::isfinite(radius) && radius >= 0.f)) return fail(ORCA_ERR_INVALID, "radius must be finite and >= 0");
+    host.assign(xy, xy + (size_t)(per_env ? s->E : 1) * num_vertices * 2);
+    for (size_t i = 0; i < host.size(); ++i)
+      if (!std::isfinite(host[i])) return fail(ORCA_ERR_INVALID, "roadmap vertex coordinates must be finite");
+  }
+  DeviceGuard guard(s->device);
+  CUDA_TRY(cudaDeviceSynchronize());  // preferred-velocity launches in flight may still read the old tables
+  s->rm_host_xy.swap(host);
+  s->rm_R = num_vertices;
+  s->rm_G = num_vertices > 0 ? num_goals : 0;
+  s->rm_per_env = num_vertices > 0 && per_env != 0;
+  s->rm_radius = radius;
+  const int rc = build_roadmap(s);
+  if (rc != ORCA_OK) {
+    s->rm_R = 0;  // no half-built roadmap
+    free_roadmap_tables(s);
+  }
+  return rc;
+}
+
+int orca_get_roadmap(const OrcaSim* s, int env, uint32_t* adjacency_out, float* dist_out) {
+  if (s == nullptr) return fail(ORCA_ERR_INVALID, "null handle");
+  if (s->rm_R == 0) return fail(ORCA_ERR_STATE, "no roadmap is set");
+  if (env < 0 || env >= s->E) return fail(ORCA_ERR_INVALID, "env %d out of range", env);
+  DeviceGuard guard(s->device);
+  const size_t t = s->rm_tables > 1 ? (size_t)env : 0;
+  const size_t words = (size_t)(s->rm_R + 31) / 32;
+  if (adjacency_out != nullptr)
+    CUDA_TRY(cudaMemcpy(adjacency_out, s->d_rm_adj + t * s->rm_R * words, (size_t)s->rm_R * words * sizeof(uint32_t),
+                        cudaMemcpyDeviceToHost));
+  if (dist_out != nullptr)
+    CUDA_TRY(cudaMemcpy(dist_out, s->d_rm_dist + t * s->rm_G * s->rm_R, (size_t)s->rm_G * s->rm_R * sizeof(float),
+                        cudaMemcpyDeviceToHost));
+  return ORCA_OK;
+}
+
+int orca_roadmap_pref_velocity(OrcaSim* s, const float* pos_dev, const int32_t* goal_vertex_dev, float* pref_dev,
+                               int32_t* vertex_out_dev, void* stream) {
+  if (s == nullptr) return fail(ORCA_ERR_INVALID, "null handle");
+  if (s->rm_R == 0) return fail(ORCA_ERR_STATE, "orca_roadmap_pref_velocity before orca_set_roadmap");
+  if (pos_dev == nullptr || goal_vertex_dev == nullptr || pref_dev == nullptr)
+    return fail(ORCA_ERR_INVALID, "orca_roadmap_pref_velocity: null pointer argument");
+  DeviceGuard guard(s->device);
+  const orca::RoadmapArgs a = roadmap_args(s);
+  const long long total = (long long)s->E * s->N;
+  const unsigned blocks = (unsigned)((total + 127) / 128);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const float2* pos = reinterpret_cast<const float2*>(pos_dev);
+  float2* pref = reinterpret_cast<float2*>(pref_dev);
+  orca::roadmap_pref_kernel<<<blocks, 128, 0, st>>>(a, s->E, s->N, pos, goal_vertex_dev, s->d_agent_params, s->p.radius,
+                                                    pref, vertex_out_dev);
+  CUDA_TRY(cudaGetLastError());
+  s->launches += 1;
   return ORCA_OK;
 }
 

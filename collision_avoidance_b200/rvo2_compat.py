@@ -13,6 +13,10 @@ Agents may have parameters of their own, as in RVO2: ``addAgent`` takes all six 
 ``Radius`` and ``MaxSpeed`` read and change them between steps.  A world whose agents all share one
 set runs the uniform kernels; a mixed one uploads its per-agent table before the next ``doStep``.
 
+``queryVisibility(point1, point2, radius)`` answers RVO2's line-of-sight query on the processed
+obstacles (True before ``processObstacles``, as in RVO2); roadmap navigation for whole batches is
+``BatchedRVOSimulator.set_roadmap`` / ``roadmap_pref_velocity``.
+
 Restrictions (checked, never silent): ``maxNeighbors <= 16``.
 """
 from __future__ import annotations
@@ -127,19 +131,23 @@ class PyRVOSimulator:
             self._params_dirty = False
         return self._sim
 
+    def _obstacle_sim(self):
+        """(simulator holding the processed obstacles, whether it is a throw-away one): with no agents
+        yet, a 1-agent world built just to run the BSP."""
+        if self._pos:
+            return self._ensure_sim(), False
+        tmp = BatchedRVOSimulator(1, 1, self._time_step, *self._defaults, device=self._device)
+        tmp.set_obstacles([p for p in self._polygons])
+        return tmp, True
+
     def _vertices(self):
         """Vertex table after processObstacles (BSP splits may have appended vertices)."""
         if self._vertex_table is None:
             if self._processed:
-                sim = self._ensure_sim() if self._pos else None
-                if sim is None:
-                    # no agents yet: build a throw-away 1-agent world just to run the BSP
-                    tmp = BatchedRVOSimulator(1, 1, self._time_step, *self._defaults, device=self._device)
-                    tmp.set_obstacles([p for p in self._polygons])
-                    self._vertex_table = tmp.obstacle_vertices(0)
-                    tmp.close()
-                else:
-                    self._vertex_table = sim.obstacle_vertices(0)
+                sim, temporary = self._obstacle_sim()
+                self._vertex_table = sim.obstacle_vertices(0)
+                if temporary:
+                    sim.close()
             else:
                 pts = np.concatenate(self._polygons) if self._polygons else np.zeros((0, 2), np.float32)
                 nxt, prv, off = [], [], 0
@@ -257,6 +265,20 @@ class PyRVOSimulator:
 
     def setAgentMaxSpeed(self, i, maxSpeed):
         self._set_param(i, 5, maxSpeed)
+
+    def queryVisibility(self, point1, point2, radius=0.0):
+        """Whether a disc of ``radius`` can move from point1 to point2 without crossing an obstacle edge
+        (RVO2's queryVisibility).  True before processObstacles: RVO2 has no obstacle tree then."""
+        if not self._processed:
+            return True
+        sim, temporary = self._obstacle_sim()
+        dev = sim.pos.device
+        q1 = torch.tensor([[[self._f32(point1[0]), self._f32(point1[1])]]], dtype=torch.float32, device=dev)
+        q2 = torch.tensor([[[self._f32(point2[0]), self._f32(point2[1])]]], dtype=torch.float32, device=dev)
+        visible = bool(sim.query_visibility(q1, q2, self._f32(radius)).item())
+        if temporary:
+            sim.close()
+        return visible
 
     def getNumAgents(self):
         return len(self._pos)

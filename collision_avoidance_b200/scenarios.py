@@ -273,6 +273,55 @@ def deadlock(num_envs: int, num_agents: int, seed: int = 0, radius: float = 0.5,
     return Scenario("deadlock", pos, vel, goal, goal2, S, polys)
 
 
+# ORCA constants of the roadmap world below (the scale of RVO2's Blocks / Roadmap examples)
+ROADMAP_PARAMS = dict(timeStep=0.25, neighborDist=15.0, maxNeighbors=10, timeHorizon=5.0, timeHorizonObst=5.0,
+                      radius=2.0, maxSpeed=2.0)
+
+
+def roadmap_blocks(num_envs: int, agents_per_group: int = 25, jitter: float = 0.0, seed: int = 0):
+    """Four square blocks around the origin, four groups of agents in the corners crossing to the
+    opposite corner, and a roadmap around the blocks -- the layout of RVO2's Blocks / Roadmap examples,
+    with numbers defined here.  Roadmap vertices: the four goals first (corner targets), then one
+    vertex off each block corner.  ``jitter`` > 0 moves every block, with its four roadmap vertices, by
+    a uniform offset in [-jitter, jitter]^2 per env: per-env obstacles and roadmaps.
+
+    Returns (Scenario, roadmap vertices float32 [R, 2] or [E, R, 2], goal vertex ids int32 [E, N])."""
+    rng = np.random.default_rng(seed)
+    goals = np.array([(-75.0, -75.0), (75.0, -75.0), (-75.0, 75.0), (75.0, 75.0)])
+    # counter-clockwise squares (RVO2's obstacle orientation) and the roadmap vertices 2 units off their corners
+    blocks_ = [np.array([(-10.0, 40.0), (-40.0, 40.0), (-40.0, 10.0), (-10.0, 10.0)]),
+               np.array([(10.0, 40.0), (10.0, 10.0), (40.0, 10.0), (40.0, 40.0)]),
+               np.array([(10.0, -40.0), (40.0, -40.0), (40.0, -10.0), (10.0, -10.0)]),
+               np.array([(-10.0, -40.0), (-10.0, -10.0), (-40.0, -10.0), (-40.0, -40.0)])]
+    corners = [b + 2.0 * np.sign(b - b.mean(0)) for b in blocks_]
+    side = int(np.ceil(np.sqrt(agents_per_group)))
+    k = np.arange(agents_per_group)
+    offs = np.stack([55.0 + 10.0 * (k % side), 55.0 + 10.0 * (k // side)], -1)
+    # group g starts in the corner opposite to goal g
+    starts = [offs * (1, 1), offs * (-1, 1), offs * (1, -1), offs * (-1, -1)]
+    pos = np.concatenate(starts)
+    goal_id = np.repeat(np.arange(4, dtype=np.int32), agents_per_group)
+    N = pos.shape[0]
+    pos = np.broadcast_to(pos, (num_envs, N, 2))
+    goal = np.broadcast_to(goals[goal_id], (num_envs, N, 2))
+    vel = np.zeros((num_envs, N, 2))
+    goal_vertex = np.ascontiguousarray(np.broadcast_to(goal_id, (num_envs, N)), np.int32)
+    if jitter > 0.0:
+        shift = rng.uniform(-jitter, jitter, size=(num_envs, 4, 1, 2))
+        worlds = [[(blocks_[b] + shift[e, b]).tolist() for b in range(4)] for e in range(num_envs)]
+        rm = np.concatenate([np.broadcast_to(goals, (num_envs, 4, 2))]
+                            + [np.asarray(corners[b]) + shift[:, b] for b in range(4)], axis=1)
+        per_env = True
+    else:
+        worlds = [b.tolist() for b in blocks_]
+        rm = np.concatenate([goals] + corners)
+        per_env = False
+    pos, vel, goal = _f32(pos, vel, goal)
+    scn = Scenario("roadmap_blocks", pos, vel, goal, goal.copy(), 150.0, worlds, per_env_obstacles=per_env,
+                   params=dict(ROADMAP_PARAMS))
+    return scn, np.ascontiguousarray(rm, np.float32), goal_vertex
+
+
 def reference_streams(seed: int, num_envs: int):
     """One ``random.Random(seed + e)`` per world: the stream the reference's module-level
     ``random.uniform`` would follow after ``random.seed(seed + e)``."""

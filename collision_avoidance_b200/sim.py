@@ -64,6 +64,7 @@ class BatchedRVOSimulator:
         self.obst_nbr_idx: Optional[torch.Tensor] = None
         self.obst_nbr_cnt: Optional[torch.Tensor] = None
         self._obst_vertex_cache = {}
+        self._roadmap_shape = None  # (R, G) of the roadmap set by set_roadmap
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -167,6 +168,82 @@ class BatchedRVOSimulator:
                                                           prv.ctypes.data, cvx.ctypes.data))
         self._obst_vertex_cache[env] = (xy, nxt, prv, cvx)
         return self._obst_vertex_cache[env]
+
+    # ------------------------------------------------------------------ line of sight and roadmaps
+    def query_visibility(self, p1: torch.Tensor, p2: torch.Tensor, radius=0.0) -> torch.Tensor:
+        """RVO2's queryVisibility for a batch: ``p1``, ``p2`` are ``[E, Q, 2]`` CUDA float32, ``radius`` a
+        float or an ``[E, Q]`` CUDA float32 tensor.  Returns a bool tensor ``[E, Q]``: whether a disc of
+        the radius moves from p1 to p2 without crossing an obstacle edge of the env's world."""
+        E = self.num_envs
+        if p1.dim() != 3 or p1.shape[0] != E or p1.shape[2] != 2:
+            raise ValueError(f"p1 must have shape [{E}, Q, 2], got {tuple(p1.shape)}")
+        Q = p1.shape[1]
+        self._check_state(p1, (E, Q, 2), torch.float32, "p1")
+        self._check_state(p2, (E, Q, 2), torch.float32, "p2")
+        r_dev, r = None, 0.0
+        if isinstance(radius, torch.Tensor):
+            self._check_state(radius, (E, Q), torch.float32, "radius")
+            r_dev = radius
+        else:
+            r = float(radius)
+        out = torch.empty(E, Q, dtype=torch.uint8, device=self.pos.device)
+        _lib.check(self._L.orca_query_visibility(self._h, self._p(p1), self._p(p2), self._p(r_dev), r, int(Q),
+                                                 self._p(out), self._stream()))
+        return out.view(torch.bool)
+
+    def set_roadmap(self, vertices, num_goals: int, radius: Optional[float] = None):
+        """Roadmap of RVO2's obstacle example (Roadmap.cpp buildRoadmap): ``vertices`` is ``[R, 2]``
+        (shared by every env) or ``[E, R, 2]`` (one roadmap per env), array or tensor; its first
+        ``num_goals`` vertices are the goals.  Edges join vertices that see each other for a disc of
+        ``radius`` (default: the constructor's radius); distances to every goal are computed on the
+        device, and again after every ``set_obstacles``.  ``R = 0`` removes the roadmap.  At most 512
+        vertices and 1 <= num_goals <= R (``NotImplementedError``).  Synchronises."""
+        if isinstance(vertices, torch.Tensor):
+            vertices = vertices.detach().cpu().numpy()
+        v = np.ascontiguousarray(np.asarray(vertices, np.float32))
+        if v.ndim == 3:
+            if v.shape[0] != self.num_envs or v.shape[2] != 2:
+                raise ValueError(f"per-env roadmap vertices must have shape [{self.num_envs}, R, 2], got {v.shape}")
+            per_env, R = True, v.shape[1]
+        elif v.ndim == 2 and v.shape[1] == 2:
+            per_env, R = False, v.shape[0]
+        else:
+            raise ValueError(f"roadmap vertices must have shape [R, 2] or [E, R, 2], got {v.shape}")
+        r = self.params.radius if radius is None else float(radius)
+        _lib.check(self._L.orca_set_roadmap(self._h, v.ctypes.data if R else None, int(R), int(num_goals),
+                                            1 if per_env else 0, r))
+        self._roadmap_shape = (R, int(num_goals)) if R else None
+
+    def roadmap(self, env: int = 0):
+        """The roadmap tables of one env: (adjacency bool [R, R], row u column v = edge u -> v;
+        distances float32 [G, R], 9e9 when unreachable)."""
+        if self._roadmap_shape is None:
+            raise RuntimeError("no roadmap is set")
+        R, G = self._roadmap_shape
+        words = (R + 31) // 32
+        adj = np.zeros((R, words), np.uint32)
+        dist = np.zeros((G, R), np.float32)
+        _lib.check(self._L.orca_get_roadmap(self._h, int(env), adj.ctypes.data, dist.ctypes.data))
+        bits = np.unpackbits(adj.view(np.uint8).reshape(R, words * 4), axis=1, bitorder="little")[:, :R]
+        return bits.astype(bool), dist
+
+    def roadmap_pref_velocity(self, goal_vertex: torch.Tensor, pos: Optional[torch.Tensor] = None,
+                              out: Optional[torch.Tensor] = None, return_vertex: bool = False):
+        """Roadmap.cpp's preferred velocities (without the perturbation) toward each agent's goal vertex
+        (``goal_vertex``: ``[E, N]`` CUDA int32, ids in [0, num_goals); others give (0, 0) and vertex -1),
+        from ``pos`` (default: the current positions).  Writes ``self.pref`` unless ``out`` is given, so
+        that ``env_step(policy=POLICY_EXTERNAL)`` / ``doStep()`` steps with it.  Returns the preferred
+        velocities, and the chosen vertex ids ``[E, N]`` int32 with ``return_vertex``."""
+        E, N = self.num_envs, self.agents_per_env
+        pos = self.pos if pos is None else pos
+        out = self.pref if out is None else out
+        self._check_state(goal_vertex, (E, N), torch.int32, "goal_vertex")
+        self._check_state(pos, (E, N, 2), torch.float32, "pos")
+        self._check_state(out, (E, N, 2), torch.float32, "out")
+        vertex = torch.empty(E, N, dtype=torch.int32, device=self.pos.device) if return_vertex else None
+        _lib.check(self._L.orca_roadmap_pref_velocity(self._h, self._p(pos), self._p(goal_vertex), self._p(out),
+                                                      self._p(vertex), self._stream()))
+        return (out, vertex) if return_vertex else out
 
     # ------------------------------------------------------------------ batched rvo2 calls
     def setAgentPosition(self, pos):

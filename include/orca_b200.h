@@ -188,6 +188,39 @@ int orca_obstacle_vertex_count(const OrcaSim* sim, int env);
 int orca_get_obstacle_vertices(const OrcaSim* sim, int env, float* xy_out, int32_t* next_out, int32_t* prev_out,
                                int32_t* convex_out);
 
+/* ---- line of sight and roadmap navigation -------------------------------------------
+ * Replaces RVO2's RVOSimulator::queryVisibility(point1, point2, radius): can a disc of `radius` move
+ * along the segment q1 -> q2 without crossing an obstacle edge?  The obstacle BSP of each query's
+ * env answers, bit for bit as RVO2's recursion does.  q1_dev, q2_dev: [E][Q][2]; radius_dev: [E][Q],
+ * or NULL for the scalar `radius` (finite, >= 0) everywhere.  visible_dev: [E][Q] bytes of 0 / 1.
+ * Every query is visible when no obstacles are set.  Asynchronous on `stream`. */
+int orca_query_visibility(OrcaSim* sim, const float* q1_dev, const float* q2_dev, const float* radius_dev,
+                          float radius, int queries_per_env, uint8_t* visible_dev, void* stream);
+/* Replaces the roadmap of RVO2's obstacle example (examples/Roadmap.cpp buildRoadmap): HOST `xy` of
+ * [W][R][2] roadmap vertices, W = 1 (shared) or W = E when `per_env` is set; the first `num_goals`
+ * vertices of each world are its goals.  Edge u -> v exists when queryVisibility(p_u, p_v, radius)
+ * (not symmetric in general); distToGoal[g][v] is Dijkstra's over those edges, weights |p_v - p_u|,
+ * 9e9f when unreachable.  Edges and distances are computed on the device for every obstacle world
+ * (per env when the obstacles or the roadmap are) and recomputed by orca_set_obstacles.  A setup
+ * call: it synchronises.  num_vertices == 0 removes the roadmap.  ORCA_ERR_UNSUPPORTED unless
+ * R <= 512 and 1 <= num_goals <= R; ORCA_ERR_INVALID for non-finite vertices or a radius that is
+ * not finite and >= 0. */
+int orca_set_roadmap(OrcaSim* sim, const float* xy, int num_vertices, int num_goals, int per_env, float radius);
+/* The roadmap tables of env `env`: adjacency as R rows of ceil(R / 32) words (row u bit v = edge
+ * u -> v), distances as [G][R].  Either output may be NULL.  Synchronises.  ORCA_ERR_STATE without a
+ * roadmap. */
+int orca_get_roadmap(const OrcaSim* sim, int env, uint32_t* adjacency_out, float* dist_out);
+/* Replaces Roadmap.cpp setPreferredVelocities (without its random perturbation) for every agent:
+ * among the roadmap vertices j with |p_j - pos| + distToGoal[goal][j] < 9e9f that are visible from
+ * the agent's position for its radius (the per-agent radius when orca_set_agent_params set one), the
+ * lowest index of smallest cost; pref = normalize(p_j - pos), or normalize(p_goal - pos) when the agent
+ * stands on a vertex other than its goal, (0, 0) on its goal or when no vertex qualifies.
+ * pos_dev [E*N][2], goal_vertex_dev [E*N] (goal ids in [0, num_goals); any other id gives pref (0, 0)
+ * and vertex -1), pref_dev [E*N][2] out, vertex_out_dev [E*N] out or NULL.  ORCA_ERR_STATE without a
+ * roadmap.  Asynchronous on `stream`. */
+int orca_roadmap_pref_velocity(OrcaSim* sim, const float* pos_dev, const int32_t* goal_vertex_dev,
+                               float* pref_dev, int32_t* vertex_out_dev, void* stream);
+
 /* ---- stepping ---------------------------------------------------------------------
  * orca_step: setAgentPrefVelocity x N + doStep (env :383-385, ALAN :598-601), batched. */
 int orca_step(OrcaSim* sim, float* pos_dev, float* vel_dev, const float* pref_dev, void* stream);
