@@ -45,6 +45,11 @@
 #define ORCA_SLOW_MAX_OBST 64
 #endif
 
+// Branch counters of host test builds (-DORCA_EMUL_COUNT); nothing at all on the device.  Slots of the LPs:
+// 0 lp3 rounds, 2 lp1 calls, 3 lp1 inner iterations, 4 projected-line fetches, 5 LP3 rounds (lp3 and
+// lp3_stored) whose projected programme was infeasible, 6 projected lines skipped as parallel in the same
+// direction, 7 antiparallel midpoints (6 and 7 per fetch: lp3 fetches a line once per access, lp3_stored
+// once per round), 8 lp3_stored rounds.
 #if defined(ORCA_EMUL_COUNT) && !defined(__CUDA_ARCH__)
 extern long long g_orca_counters[16];
 #define ORCA_COUNT(slot, n) (g_orca_counters[slot] += (n))
@@ -302,7 +307,11 @@ struct ProjectedLines {
     const float d = det(di, dj);
     float2 np;
     if (fabsf(d) <= kEps) {
-      if (dot(di, dj) > 0.f) return false;
+      if (dot(di, dj) > 0.f) {
+        ORCA_COUNT(6, 1);  // parallel, same direction: no line
+        return false;
+      }
+      ORCA_COUNT(7, 1);  // antiparallel: midpoint
       np = mul(0.5f, add(pi, pj));
     } else {
       np = add(pi, mul(det(dj, sub(pi, pj)) / d, di));
@@ -346,6 +355,7 @@ ORCA_HD void lp3(unsigned mask, bool need, const LS& L, int n, int n_obst, int b
     float2 cand = result;
     const int f = lp2(mask, active, V, m, radius, v2(-V.di.y, V.di.x), true, cand);
     if (active) {
+      if (f < m) ORCA_COUNT(5, 1);  // infeasible projected programme
       if (!(f < m)) result = cand;  // on failure keep the previous result
       distance = det(V.di, sub(V.pi, result));
       ++i;
@@ -373,6 +383,7 @@ ORCA_HD void lp3_stored(unsigned mask, bool need, const LS& L, int n, int n_obst
         ++i;
       }
       active = i < n;
+      if (active) ORCA_COUNT(8, 1);  // lp3_stored rounds
     }
     ORCA_CONVERGE(mask);
     int m = 0;
@@ -392,6 +403,7 @@ ORCA_HD void lp3_stored(unsigned mask, bool need, const LS& L, int n, int n_obst
     float2 cand = result;
     const int f = lp2(mask, active, P, m, radius, v2(-di.y, di.x), true, cand);
     if (active) {
+      if (f < m) ORCA_COUNT(5, 1);  // infeasible projected programme
       if (!(f < m)) result = cand;  // on failure keep the previous result
       distance = det(di, sub(pi, result));
       ++i;
