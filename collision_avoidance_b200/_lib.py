@@ -29,6 +29,8 @@ STAT_SUM_ARRIVAL, STAT_SUM_ARRIVAL2, STAT_SUM_REWARD, STAT_COUNT = 5, 6, 7, 8
 HOST_UPLOAD_STATE, HOST_AUX_UNCHANGED = 1, 2
 
 MAX_OBST_NEIGHBORS = 16
+MAX_OBST_LINES = 6         # obstacle lines of the step's fast path (orca_b200.h ORCA_MAX_OBST_LINES)
+SLOW_MAX_OBST = 64         # obstacle lines the uncapped path holds (ORCA_SLOW_MAX_OBST)
 MAX_ACTIONS = 16
 
 # every symbol include/orca_b200.h declares (tests check the .so exports all of them)
@@ -36,7 +38,7 @@ EXPORTED_SYMBOLS = (
     "orca_abi_version", "orca_last_error", "orca_create", "orca_destroy", "orca_get_params", "orca_set_agent_params",
     "orca_set_obstacles", "orca_obstacle_vertex_count", "orca_get_obstacle_vertices",
     "orca_query_visibility", "orca_set_roadmap", "orca_get_roadmap", "orca_roadmap_pref_velocity",
-    "orca_step", "orca_env_step", "orca_env_step_many", "orca_neighbors", "orca_observe", "orca_step_host", "orca_step_host_ex", "orca_policy_mlp", "orca_policy_mlp_fp32", "orca_launch_count",
+    "orca_step", "orca_env_step", "orca_env_step_many", "orca_neighbors", "orca_agent_lines", "orca_observe", "orca_step_host", "orca_step_host_ex", "orca_policy_mlp", "orca_policy_mlp_fp32", "orca_launch_count",
 )
 
 
@@ -140,6 +142,7 @@ def load() -> ctypes.CDLL:
     L.orca_env_step.argtypes = [hp, ctypes.POINTER(OrcaEnvStepArgs), _vp]
     L.orca_env_step_many.argtypes = [hp, ctypes.POINTER(OrcaEnvStepArgs), i, _vp]
     L.orca_neighbors.argtypes = [hp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
+    L.orca_agent_lines.argtypes = [hp, _vp, _vp, i, _vp, _vp, _vp, _vp]
     L.orca_observe.argtypes = [hp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, i, i, _vp, _vp]
     L.orca_step_host.argtypes = [hp, _vp, _vp, _vp, i, i, i]
     L.orca_step_host_ex.argtypes = [hp, _vp, _vp, _vp, i, i, i]

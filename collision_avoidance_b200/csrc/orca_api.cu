@@ -21,6 +21,7 @@
 #include "obstacle_world.h"
 #include "orca_core.cuh"
 #include "orca_grid.cuh"
+#include "orca_lines.cuh"
 #include "orca_obs.cuh"
 #include "orca_policy.cuh"
 #include "orca_policy_tc.cuh"
@@ -129,6 +130,8 @@ struct OrcaSim {
   float* d_rm_dist = nullptr;
   // uniform-grid scratch (large worlds)
   orca::GridScratch grid;
+  // ... of orca_agent_lines: a set of its own, so that the query never writes what a step reads
+  orca::GridScratch lines_grid;
   int64_t launches = 0;
 };
 
@@ -426,6 +429,48 @@ int ensure_host_staging(OrcaSim* s) {
   return ORCA_OK;
 }
 
+template <int K>
+int launch_agent_lines(OrcaSim* s, const orca::StepArgs& a, const orca::LinesOut& o, cudaStream_t st) {
+  const float4* params = s->d_agent_params;
+  if (s->N >= s->grid_min_agents) {
+    // G1-G4 into the query's own grid scratch, without the step-counter bump: nothing a step reads
+    // (the step's scratch, the neighbor-search hint, the step counters) is written, so the call needs
+    // no ordering against steps -- only against whatever writes pos / vel, and against other
+    // orca_agent_lines calls on the handle (they share this scratch)
+    orca::GridScratch& G = s->lines_grid;
+    const int rc = orca::grid_prep(G, a, 0, st, &g_last_error);
+    if (rc != 0) return rc;
+    const int T = s->E * s->N;
+    const int tpb = orca::kLinesGridThreads;
+    const size_t smem = (size_t)(K + ORCA_MAX_OBST_LINES) * tpb * sizeof(float4);
+    auto kern = orca::agent_lines_grid_kernel<K>;
+    static std::atomic<bool> attr_set[orca::kMaxDevices];  // function attributes are per device
+    if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
+      CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
+    }
+    kern<<<(T + tpb - 1) / tpb, tpb, smem, st>>>(a, G.sorted_pv, G.sorted_idx, G.cell_start, G.params, params, o);
+    CUDA_TRY(cudaGetLastError());
+    s->launches += orca::kGridLaunchesPerStep;
+    return ORCA_OK;
+  }
+  const int tpb = orca::kLinesTileThreads;
+  orca::StepArgs args = a;
+  args.envs_per_block = tpb / s->N;
+  const int blocks = (s->E + args.envs_per_block - 1) / args.envs_per_block;
+  const size_t smem = orca::lines_tile_smem_bytes(tpb);
+  auto kern = orca::agent_lines_tile_kernel<K>;
+  static std::atomic<bool> attr_set[orca::kMaxDevices];
+  if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
+    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
+  }
+  kern<<<blocks, tpb, smem, st>>>(args, params, o);
+  CUDA_TRY(cudaGetLastError());
+  s->launches += 1;
+  return ORCA_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -486,6 +531,7 @@ int orca_destroy(OrcaSim* s) {
   }
   if (s->host_fork) cudaEventDestroy(s->host_fork);
   orca::grid_free(s->grid);
+  orca::grid_free(s->lines_grid);
   delete s;
   return ORCA_OK;
 }
@@ -853,6 +899,32 @@ int orca_neighbors(OrcaSim* s, const float* pos_dev, int32_t* nbr_idx_dev, float
   a.onbr_cnt = obst_nbr_cnt_dev;
   a.neighbors_only = 1;
   return launch_step(s, a, ORCA_POLICY_EXTERNAL, static_cast<cudaStream_t>(stream));
+}
+
+int orca_agent_lines(OrcaSim* s, const float* pos_dev, const float* vel_dev, int max_lines, float* lines_dev,
+                     int32_t* line_cnt_dev, int32_t* obst_line_cnt_dev, void* stream) {
+  if (s == nullptr) return fail(ORCA_ERR_INVALID, "null handle");
+  if (pos_dev == nullptr || vel_dev == nullptr || line_cnt_dev == nullptr)
+    return fail(ORCA_ERR_INVALID, "orca_agent_lines: pos_dev, vel_dev and line_cnt_dev are required");
+  if (max_lines < 0) return fail(ORCA_ERR_INVALID, "max_lines must be >= 0");
+  if (max_lines > 0 && lines_dev == nullptr) return fail(ORCA_ERR_INVALID, "orca_agent_lines: lines_dev is required when max_lines > 0");
+  DeviceGuard guard(s->device);
+  orca::StepArgs a;
+  fill_common(s, &a);  // no nbr_hint, env_step or stats: nothing a later step reads is written
+  a.pos = reinterpret_cast<float2*>(const_cast<float*>(pos_dev));
+  a.vel = reinterpret_cast<float2*>(const_cast<float*>(vel_dev));
+  a.neighbors_only = 1;
+  if (s->d_agent_params != nullptr) a.nd_sq = s->max_nd * s->max_nd;  // the grid's cell size, as in launch_step
+  orca::LinesOut o;
+  o.lines = reinterpret_cast<float4*>(lines_dev);
+  o.cnt = line_cnt_dev;
+  o.obst_cnt = obst_line_cnt_dev;
+  o.max_lines = max_lines;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int K = pick_k(s->p.max_neighbors);
+  if (K == 5) return launch_agent_lines<5>(s, a, o, st);
+  if (K == 10) return launch_agent_lines<10>(s, a, o, st);
+  return launch_agent_lines<16>(s, a, o, st);
 }
 
 int orca_observe(OrcaSim* s, const float* pos_dev, const float* vel_dev, const float* goal_dev, const int32_t* nbr_idx_dev,

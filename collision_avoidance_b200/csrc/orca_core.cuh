@@ -49,7 +49,7 @@
 // 0 lp3 rounds, 2 lp1 calls, 3 lp1 inner iterations, 4 projected-line fetches, 5 LP3 rounds (lp3 and
 // lp3_stored) whose projected programme was infeasible, 6 projected lines skipped as parallel in the same
 // direction, 7 antiparallel midpoints (6 and 7 per fetch: lp3 fetches a line once per access, lp3_stored
-// once per round), 8 lp3_stored rounds.
+// once per round), 8 lp3_stored rounds, 9 obstacle edges skipped as already covered (obstacle_lines).
 #if defined(ORCA_EMUL_COUNT) && !defined(__CUDA_ARCH__)
 extern long long g_orca_counters[16];
 #define ORCA_COUNT(slot, n) (g_orca_counters[slot] += (n))
@@ -848,7 +848,7 @@ ORCA_HD int obstacle_lines(const ObstacleWorld& W, float2 p, float2 vel, float r
         break;
       }
     }
-    if (covered) continue;
+    if (covered) { ORCA_COUNT(9, 1); continue; }  // (host test builds count the edges skipped as covered)
 
     const float d1 = abs_sq(rp1), d2 = abs_sq(rp2);
     const float2 ov = sub(p2, p1);

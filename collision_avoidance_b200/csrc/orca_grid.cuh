@@ -616,9 +616,12 @@ inline int grid_ensure(GridScratch& G, const StepArgs& a, cudaStream_t st, std::
 
 constexpr int kGridLaunchesPerStep = 5;  // G1 bounds, G2 count, G3 scan, G4 scatter, G5 step
 
-template <int K, bool KFULL, int POLICY, int OL, bool HETERO = false>
-int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t* launches, std::string* err,
-                    const float4* agent_params = nullptr) {
+// G1-G4: the cell-sorted snapshot of (a.pos, a.vel) in G.  `bump`: G2 also bumps the env step counters
+// (a.env_step, when given).  Any number of runs may follow each other on one stream: the accumulators
+// re-arm themselves, the scan re-zeroes the counts it read and tags its tile states with a fresh epoch.
+// Runs on the same GridScratch from two streams at once would race; orca_agent_lines has a scratch of
+// its own, orca_neighbors uses the step's and is ordered with the steps by the caller's stream.
+inline int grid_prep(GridScratch& G, const StepArgs& a, int bump, cudaStream_t st, std::string* err) {
   const int T = a.E * a.N;
   const int rc = grid_ensure(G, a, st, err);
   if (rc != 0) return rc;
@@ -626,13 +629,22 @@ int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t*
   const int nb_agents = (T + tpb - 1) / tpb;
   grid_bounds_kernel<<<G.sm_count * 2, kBoundsThreads, 0, st>>>(a.pos, T, G.counters, sqrtf(a.nd_sq), a.E, G.cap_cells, G.params);
   grid_count_kernel<<<nb_agents, tpb, 0, st>>>(a.pos, T, a.N, G.params, G.cell_count, G.key, G.slot, a.env_step,
-                                               a.env_done_cnt, G.env_step_snap, a.E, a.neighbors_only ? 0 : 1);
+                                               a.env_done_cnt, G.env_step_snap, a.E, bump);
   const int scan_blocks = (G.cap_cells + kScanTile - 1) / kScanTile;
   G.epoch = (G.epoch + 1u) & 0x3fffffffu;
   if (G.epoch == 0u) G.epoch = 1u;  // 0 is the state of freshly cleared words
   grid_scan_kernel<<<scan_blocks, kScanThreads, 0, st>>>(G.cell_count, G.params, G.tile_state, G.counters + 5, G.epoch,
                                                         G.cell_start);
   grid_scatter_kernel<<<nb_agents, tpb, 0, st>>>(a.pos, a.vel, T, G.key, G.slot, G.cell_start, G.sorted_pv, G.sorted_idx);
+  return 0;
+}
+
+template <int K, bool KFULL, int POLICY, int OL, bool HETERO = false>
+int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t* launches, std::string* err,
+                    const float4* agent_params = nullptr) {
+  const int T = a.E * a.N;
+  const int rc = grid_prep(G, a, a.neighbors_only ? 0 : 1, st, err);
+  if (rc != 0) return rc;
   StepArgs args = a;
   // the step kernel only READS the step counters in this path, from the copy G2 made
   const int stpb = ORCA_GRID_TPB;

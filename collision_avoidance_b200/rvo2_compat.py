@@ -13,6 +13,12 @@ Agents may have parameters of their own, as in RVO2: ``addAgent`` takes all six 
 ``Radius`` and ``MaxSpeed`` read and change them between steps.  A world whose agents all share one
 set runs the uniform kernels; a mixed one uploads its per-agent table before the next ``doStep``.
 
+``getAgentNumORCALines(i)`` / ``getAgentORCALine(i, j)`` return the ORCA half-planes agent i solved in
+the last ``doStep``, as in RVO2.  They are computed on the first query after a step (from the pre-step
+state the shim keeps), so ``doStep`` costs nothing more for callers that never ask; a call that would
+change what the device computes (``addAgent``, ``addObstacle``, ``processObstacles``, a ``setAgent*``
+parameter setter) computes them first.
+
 ``queryVisibility(point1, point2, radius)`` answers RVO2's line-of-sight query on the processed
 obstacles (True before ``processObstacles``, as in RVO2); roadmap navigation for whole batches is
 ``BatchedRVOSimulator.set_roadmap`` / ``roadmap_pref_velocity``.
@@ -50,6 +56,10 @@ class PyRVOSimulator:
         self._sim: Optional[BatchedRVOSimulator] = None
         self._dirty = True            # host state newer than device state
         self._nbr_host = None         # (nbr_idx, nbr_cnt, obst_idx, obst_cnt) of the last doStep
+        # ORCA lines of the last doStep: its pre-step (pos, vel) until the first query or mutation, then
+        # the host copy (lines [n, L, 4], count [n], n_obst [n]) for the n agents the step had
+        self._lines_pending = None
+        self._lines_host = None
         self._global_time = 0.0
         self._vertex_table = None
 
@@ -65,6 +75,7 @@ class PyRVOSimulator:
             params = (float(neighborDist), int(maxNeighbors), float(timeHorizon), float(timeHorizonObst),
                       float(radius), float(maxSpeed))
             vel = (float(velocity[0]), float(velocity[1]))
+        self._materialize_lines()
         self._params.append(tuple(self._f32(x) if i != 1 else x for i, x in enumerate(params)))
         self._params_dirty = True
         self._pos.append((float(np.float32(pos[0])), float(np.float32(pos[1]))))
@@ -78,6 +89,7 @@ class PyRVOSimulator:
         arr = np.asarray(vertices, dtype=np.float32).reshape(-1, 2)
         if arr.shape[0] < 2:
             raise RuntimeError("Error adding obstacle to RVO simulation")
+        self._materialize_lines()
         first = sum(p.shape[0] for p in self._polygons)
         self._polygons.append(arr)
         self._processed = False
@@ -85,6 +97,7 @@ class PyRVOSimulator:
         return first
 
     def processObstacles(self):
+        self._materialize_lines()
         self._processed = True
         self._vertex_table = None
         if self._sim is not None:
@@ -106,6 +119,8 @@ class PyRVOSimulator:
     def _ensure_sim(self) -> BatchedRVOSimulator:
         if not self._pos:
             raise RuntimeError("no agents in the simulation")
+        if self._params_dirty:
+            self._materialize_lines()  # the last step's lines come from the parameters it ran with
         hp, hetero = self._handle_params()
         if self._sim is not None and hp != self._sim_params:
             self._sim = None  # another maxNeighbors bound (or another shared set): rebuild
@@ -167,6 +182,9 @@ class PyRVOSimulator:
             sim.vel.copy_(torch.tensor(self._vel, dtype=torch.float32).reshape(1, -1, 2))
         sim.pref.copy_(torch.tensor(self._pref, dtype=torch.float32).reshape(1, -1, 2))
         sim.env_step(policy=_lib.POLICY_EXTERNAL, want_neighbors=True, collect_stats=False)
+        # the host lists are replaced below, never changed in place: they stay this step's input
+        self._lines_pending = (self._pos, self._vel)
+        self._lines_host = None
         pos = sim.pos[0].cpu().numpy()
         vel = sim.vel[0].cpu().numpy()
         self._pos = [(float(p[0]), float(p[1])) for p in pos]
@@ -213,6 +231,44 @@ class PyRVOSimulator:
             raise IndexError("neighbor index out of range")
         return int(self._nbr_host[2][i, j])
 
+    def _materialize_lines(self):
+        """Compute the ORCA lines of the last doStep from its kept pre-step state, on the simulator
+        (parameters, obstacles) it ran with."""
+        if self._lines_pending is None:
+            return
+        pos, vel = self._lines_pending
+        self._lines_pending = None
+        sim = self._sim
+        dev = sim.pos.device
+        p = torch.tensor(pos, dtype=torch.float32, device=dev).reshape(1, -1, 2)
+        v = torch.tensor(vel, dtype=torch.float32, device=dev).reshape(1, -1, 2)
+        lines, count, n_obst = sim.orca_lines(p, v, max_lines=sim.max_neighbors + _lib.SLOW_MAX_OBST)
+        self._lines_host = (lines[0].cpu().numpy(), count[0].cpu().numpy(), n_obst[0].cpu().numpy())
+
+    def _num_lines(self, i):
+        self._materialize_lines()
+        if self._lines_host is None or i >= self._lines_host[1].shape[0]:
+            return 0  # before the first doStep, or an agent added after it
+        n = int(self._lines_host[1][i])
+        if n < 0:
+            raise RuntimeError(f"agent {i} has more than {_lib.SLOW_MAX_OBST} obstacle lines")
+        return n
+
+    def getAgentNumORCALines(self, i):
+        """Number of ORCA half-planes agent i solved in the last doStep (0 before the first one)."""
+        if not 0 <= i < len(self._pos):
+            raise IndexError("agent index out of range")
+        return self._num_lines(i)
+
+    def getAgentORCALine(self, i, j):
+        """Half-plane j of agent i in the last doStep as (point.x, point.y, direction.x, direction.y):
+        obstacle lines first, then agent lines by ascending distance.  The flat tuple follows
+        Python-RVO2's rvo2.pyx as far as it is known without its source at hand; the test suite pins it."""
+        if not 0 <= i < len(self._pos) or not 0 <= j < self._num_lines(i):
+            raise IndexError("ORCA line index out of range")
+        ln = self._lines_host[0][i, j]
+        return (float(ln[0]), float(ln[1]), float(ln[2]), float(ln[3]))
+
     def getNextObstacleVertexNo(self, v):
         return int(self._vertices()[1][v])
 
@@ -225,6 +281,7 @@ class PyRVOSimulator:
 
     # per-agent parameters (RVO2's getAgent* / setAgent*); a change takes effect at the next doStep
     def _set_param(self, i, j, value):
+        self._materialize_lines()
         p = list(self._params[i])
         p[j] = int(value) if j == 1 else self._f32(value)
         self._params[i] = tuple(p)

@@ -290,6 +290,37 @@ class BatchedRVOSimulator:
         out = (self.nbr_idx, self.nbr_cnt, self.obst_nbr_idx, self.obst_nbr_cnt)
         return out + (dsq,) if with_distsq else out
 
+    def orca_lines(self, pos: Optional[torch.Tensor] = None, vel: Optional[torch.Tensor] = None,
+                   max_lines: Optional[int] = None):
+        """The ORCA half-planes every agent solves in the NEXT step from the state ``(pos, vel)``
+        (default: the current ``self.pos`` / ``self.vel``) -- RVO2's getAgentNumORCALines /
+        getAgentORCALine for the whole batch.  To record what a step solves, call this before stepping.
+
+        Returns device tensors ``(lines [E, N, L, 4] float32, count [E, N] int32, n_obst [E, N] int32)``.
+        Row ``j`` of an agent is ``(point.x, point.y, direction.x, direction.y)``: its ``n_obst`` obstacle
+        lines first, then one line per agent neighbor in ascending (distSq, id) order, bit for bit the
+        programme of the step.  ``L = max_lines`` (default ``maxNeighbors + 6``, the obstacle lines of the
+        step's fast path); rows past ``L`` are absent, which ``count > L`` shows, and rows at and past
+        ``count`` are zero.  ``count = -1``: more than 64 obstacle lines (the step's overflow statistic).
+        The lines do not depend on the preferred velocity.  Writes nothing a step reads."""
+        E, N = self.num_envs, self.agents_per_env
+        pos = self.pos if pos is None else pos
+        vel = self.vel if vel is None else vel
+        self._check_state(pos, (E, N, 2), torch.float32, "pos")
+        self._check_state(vel, (E, N, 2), torch.float32, "vel")
+        if pos.device != self.pos.device or vel.device != self.pos.device:
+            raise ValueError(f"pos and vel must live on {self.pos.device}")
+        L = self.max_neighbors + _lib.MAX_OBST_LINES if max_lines is None else int(max_lines)
+        if L < 0:
+            raise ValueError(f"max_lines must be >= 0, got {L}")
+        dev = self.pos.device
+        lines = torch.zeros(E, N, L, 4, dtype=torch.float32, device=dev)
+        count = torch.empty(E, N, dtype=torch.int32, device=dev)
+        n_obst = torch.empty(E, N, dtype=torch.int32, device=dev)
+        _lib.check(self._L.orca_agent_lines(self._h, self._p(pos), self._p(vel), L, self._p(lines) if L else None,
+                                            self._p(count), self._p(n_obst), self._stream()))
+        return lines, count, n_obst
+
     # ------------------------------------------------------------------ fused env step
     def env_step(self, *, policy: int, goal: Optional[torch.Tensor] = None, goal2: Optional[torch.Tensor] = None,
                  done_mode: int = _lib.DONE_NONE, action_theta: Optional[torch.Tensor] = None,

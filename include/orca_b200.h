@@ -236,6 +236,21 @@ int orca_env_step_many(OrcaSim* sim, const OrcaEnvStepArgs* args, int steps, voi
 int orca_neighbors(OrcaSim* sim, const float* pos_dev, int32_t* nbr_idx_dev, float* nbr_distsq_dev,
                    int32_t* nbr_cnt_dev, int32_t* obst_nbr_idx_dev, int32_t* obst_nbr_cnt_dev, void* stream);
 
+/* The ORCA half-planes every agent would solve in a step from (pos, vel): RVO2's
+ * getAgentNumORCALines / getAgentORCALine.  Obstacle lines first (RVO2's order, covered edges
+ * skipped), then one line per agent neighbor in ascending (distSq, id); each line is (point.x, point.y,
+ * direction.x, direction.y), bit for bit what the next orca_step / orca_env_step from this state
+ * solves (the preferred velocity plays no part).  lines_dev [E*N][max_lines][4]; rows past max_lines
+ * are not written, counts are always complete.  line_cnt_dev [E*N] (-1: beyond the uncapped capacity,
+ * ORCA_SLOW_MAX_OBST obstacle lines), obst_line_cnt_dev [E*N] or NULL.  max_lines = 0 gives counts
+ * only.  Writes nothing a step reads (no neighbor-search hint, step counter, statistic or step scratch):
+ * on worlds of more than 256 agents it sorts (pos, vel) into a grid scratch of its own (allocated at the
+ * first such call, about 36 B per agent plus the cells).  Asynchronous on `stream`: order it after
+ * whatever writes pos_dev / vel_dev, and order two orca_agent_lines calls on one handle (they share that
+ * scratch). */
+int orca_agent_lines(OrcaSim* sim, const float* pos_dev, const float* vel_dev, int max_lines, float* lines_dev,
+                     int32_t* line_cnt_dev, int32_t* obst_line_cnt_dev, void* stream);
+
 /* Laser-scan observation of every agent: Collision_Avoidance_Env._get_obs + utils.comp_laser
  * (collision_avoidence_env.py:231-350 ; utils.py:5-113).  `laser_num` rays of length
  * neighbor_dist per agent, neighbors approximated by `circle_approx_num`-gons of the agent
