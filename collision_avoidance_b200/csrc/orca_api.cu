@@ -19,6 +19,7 @@
 
 #include "../../include/orca_b200.h"
 #include "obstacle_world.h"
+#include "step_plan.h"
 #include "orca_core.cuh"
 #include "orca_grid.cuh"
 #include "orca_lines.cuh"
@@ -161,11 +162,31 @@ void free_obstacles(OrcaSim* s) {
   s->worlds.clear();
 }
 
-int pick_k(int k) {
-  if (k <= 5) return 5;
-  if (k <= 10) return 10;
-  if (k <= 16) return 16;
-  return -1;
+orca_host::StepPlan step_plan_of(const OrcaSim* s) {
+  orca_host::StepPlanInputs in;
+  in.N = s->N;
+  in.max_neighbors = s->p.max_neighbors;
+  in.grid_min_agents = s->grid_min_agents;
+  in.vert_stride = s->vert_stride;
+  in.per_env = s->per_env;
+  in.hetero = s->d_agent_params != nullptr;
+  in.no_slim = std::getenv("ORCA_B200_NO_SLIM_KERNEL") != nullptr;  // dev knob
+  return orca_host::step_plan(in);
+}
+
+// Function attributes are per device: one flag per (kernel, device).  Distinct handles may be driven
+// from distinct threads: atomic flags; setting an attribute twice is harmless.
+constexpr int kMaxDevices = 64;
+template <auto Kern>
+cudaError_t set_attrs_once(int device, int max_smem, bool max_carveout) {
+  static std::atomic<bool> attr_set[kMaxDevices];
+  if (device < kMaxDevices && attr_set[device].load(std::memory_order_acquire)) return cudaSuccess;
+  cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+  // the whole unified L1 as shared memory: the resident-block count is what the step kernels live on
+  if (e == cudaSuccess && max_carveout)
+    e = cudaFuncSetAttribute(Kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
+  if (e == cudaSuccess && device < kMaxDevices) attr_set[device].store(true, std::memory_order_release);
+  return e;
 }
 
 void fill_common(const OrcaSim* s, orca::StepArgs* a) {
@@ -195,8 +216,41 @@ void fill_common(const OrcaSim* s, orca::StepArgs* a) {
   a->cull_geo = s->d_cull_geo;
 }
 
-template <int K, bool KFULL, int POLICY, int OL, bool HETERO = false>
-int launch_small_kpo(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
+// The tile and the grid step kernel of one instantiation, each with its attribute setter.
+using TileKernel = decltype(&orca::step_small_kernel<5, true, orca::POLICY_EXTERNAL>);
+using GridKernel = decltype(&orca::step_grid_kernel<5, true, orca::POLICY_EXTERNAL>);
+struct StepKernels {
+  TileKernel tile;
+  cudaError_t (*tile_attrs)(int device, int max_smem, bool max_carveout);
+  GridKernel grid;
+  cudaError_t (*grid_attrs)(int device, int max_smem, bool max_carveout);
+};
+
+template <int K, bool KFULL, int POLICY, int OL, bool HETERO>
+StepKernels kernels_of() {
+  constexpr TileKernel tile = orca::step_small_kernel<K, KFULL, POLICY, OL, HETERO>;
+  constexpr GridKernel grid = orca::step_grid_kernel<K, KFULL, POLICY, OL, HETERO>;
+  return {tile, set_attrs_once<tile>, grid, set_attrs_once<grid>};
+}
+
+// The (K, KFULL, OL, HETERO) combinations step_plan produces: K = 5 / 10 / 16, the slim 10, and the
+// per-agent-parameter K = 5 / 10 / 16.
+template <int POLICY>
+StepKernels kernels_for(const orca_host::StepPlan& p) {
+  constexpr int OL = ORCA_MAX_OBST_LINES;
+  if (p.hetero) {
+    if (p.K == 5) return kernels_of<5, false, POLICY, OL, true>();
+    if (p.K == 10) return kernels_of<10, false, POLICY, OL, true>();
+    return kernels_of<16, false, POLICY, OL, true>();
+  }
+  if (p.ol == 2) return kernels_of<10, true, POLICY, 2, false>();
+  if (p.K == 5) return kernels_of<5, true, POLICY, OL, false>();
+  if (p.K == 10) return kernels_of<10, true, POLICY, OL, false>();
+  return kernels_of<16, false, POLICY, OL, false>();
+}
+
+int launch_tile_step(OrcaSim* s, const orca::StepArgs& a, const orca_host::StepPlan& p, const StepKernels& k,
+                     cudaStream_t st) {
   const int N = s->N;
   // 256-thread blocks: whole envs per block (256 / N of them); measured faster than 128 / 64 / 32
   // because the block-level LP3 queue gets denser (DESIGN.md section 5)
@@ -214,86 +268,42 @@ int launch_small_kpo(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
   // worlds of more than 32 agents: candidates come from an in-block uniform grid (cell = neighborDist + 0.1 %)
   args.tile_grid_inv_cell = 0.f;
   // (per-agent parameters: the largest neighborDist of the table)
-  const float nd = HETERO ? s->max_nd : s->p.neighbor_dist;
+  const float nd = p.hetero ? s->max_nd : s->p.neighbor_dist;
   if (N > 32 && nd > 0.f && std::getenv("ORCA_B200_NO_TILE_GRID") == nullptr)
     args.tile_grid_inv_cell = 1.0f / (nd * 1.001f);
-  size_t smem = orca::step_smem_bytes(K, tpb, true, args.world_slots, OL, HETERO);
-  auto kern = orca::step_small_kernel<K, KFULL, POLICY, OL, HETERO>;
-  // function attributes are per device: one flag per (instantiation, device)
-  // (distinct handles may be driven from distinct threads: atomic flags; setting the attribute twice is harmless)
-  static std::atomic<bool> attr_set[orca::kMaxDevices];
-  if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
-    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)orca::step_smem_bytes(K, 256, true, 256, OL, HETERO)));
-    // the whole unified L1 as shared memory: the resident-block count is what this kernel lives on
-    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
-  }
+  size_t smem = orca::step_smem_bytes(p.K, tpb, true, args.world_slots, p.ol, p.hetero);
+  // the largest size any launch of this kernel asks for
+  CUDA_TRY(k.tile_attrs(s->device, (int)orca::step_smem_bytes(p.K, 256, true, 256, p.ol, p.hetero), true));
   if (const char* e = std::getenv("ORCA_B200_SMEM_PAD")) {  // dev knob: extra shared memory = fewer resident blocks (occupancy experiments)
     const long v = std::atol(e);
     if (v > 0 && smem + (size_t)v <= 227 * 1024) {
       smem += (size_t)v;
-      CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      CUDA_TRY(cudaFuncSetAttribute(k.tile, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
   }
-  kern<<<blocks, tpb, smem, st>>>(args, HETERO ? s->d_agent_params : nullptr);
+  k.tile<<<blocks, tpb, smem, st>>>(args, s->d_agent_params);
   CUDA_TRY(cudaGetLastError());
   s->launches += 1;
   return ORCA_OK;
 }
 
-template <int K, bool KFULL, int POLICY>
-int launch_small_kp(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
-  // a world of at most 4 processed vertices (none, or one wall) gives an agent at most 2 obstacle lines:
-  // the K + 2 slot kernel, four blocks per SM (see step_small_kernel).  Instantiated for K = 10 (the ALAN
-  // shells' maxNeighbors: BASELINE configs 2 and 3) only.
-  // (worlds of more than 32 agents search through the candidate buffer, which lives in the line slots:
-  // with 12 instead of 16 of them the smaller buffer costs more than the fourth block gains -- measured
-  // 509 vs 501 us for 50-agent crowds, 497 vs 492 us for 256-agent crowds)
-  if (K == 10 && s->vert_stride <= 4 && s->N <= 32 && std::getenv("ORCA_B200_NO_SLIM_KERNEL") == nullptr)
-    return launch_small_kpo<10, true, POLICY, 2>(s, a, st);
-  return launch_small_kpo<K, KFULL, POLICY, ORCA_MAX_OBST_LINES>(s, a, st);
-}
-
-template <int K, bool KFULL>
-int launch_small_k(OrcaSim* s, const orca::StepArgs& a, int policy, cudaStream_t st) {
-  switch (policy) {
-    case ORCA_POLICY_EXTERNAL:
-      return launch_small_kp<K, KFULL, orca::POLICY_EXTERNAL>(s, a, st);
-    case ORCA_POLICY_GOAL:
-      return launch_small_kp<K, KFULL, orca::POLICY_GOAL>(s, a, st);
-    case ORCA_POLICY_RL:
-      return launch_small_kp<K, KFULL, orca::POLICY_RL>(s, a, st);
-    case ORCA_POLICY_ALAN:
-      return launch_small_kp<K, KFULL, orca::POLICY_ALAN>(s, a, st);
-    default:
-      return fail(ORCA_ERR_INVALID, "unknown policy %d", policy);
-  }
-}
-
-// Per-agent parameters: the HETERO variants of the full tile kernel and of the grid kernel, K from the
-// handle's maxNeighbors (the width of the neighbor-list rows), lists of KFULL = false (per-agent k <= K).
-template <int K, int POLICY>
-int launch_hetero_kp(OrcaSim* s, const orca::StepArgs& a, cudaStream_t st) {
-  if (s->N >= s->grid_min_agents)
-    return orca::launch_grid_kpo<K, false, POLICY, ORCA_MAX_OBST_LINES, true>(s->grid, a, st, &s->launches, &g_last_error,
-                                                                              s->d_agent_params);
-  return launch_small_kpo<K, false, POLICY, ORCA_MAX_OBST_LINES, true>(s, a, st);
-}
-
-template <int K>
-int launch_hetero_k(OrcaSim* s, const orca::StepArgs& a, int policy, cudaStream_t st) {
-  switch (policy) {
-    case ORCA_POLICY_EXTERNAL:
-      return launch_hetero_kp<K, orca::POLICY_EXTERNAL>(s, a, st);
-    case ORCA_POLICY_GOAL:
-      return launch_hetero_kp<K, orca::POLICY_GOAL>(s, a, st);
-    case ORCA_POLICY_RL:
-      return launch_hetero_kp<K, orca::POLICY_RL>(s, a, st);
-    case ORCA_POLICY_ALAN:
-      return launch_hetero_kp<K, orca::POLICY_ALAN>(s, a, st);
-    default:
-      return fail(ORCA_ERR_INVALID, "unknown policy %d", policy);
-  }
+// G1-G4 into the step's grid scratch (G2 bumps the step counters unless the call only searches), then G5.
+int launch_grid_step(OrcaSim* s, const orca::StepArgs& a, const orca_host::StepPlan& p, const StepKernels& k,
+                     cudaStream_t st) {
+  orca::GridScratch& G = s->grid;
+  const int rc = orca::grid_prep(G, a, a.neighbors_only ? 0 : 1, st, &g_last_error);
+  if (rc != ORCA_OK) return rc;
+  const int T = a.E * a.N;
+  const int tpb = ORCA_GRID_TPB;
+  const size_t smem = orca::step_smem_bytes(p.K, tpb, false, 0, p.ol, p.hetero);
+  CUDA_TRY(k.grid_attrs(s->device, (int)smem, true));
+  orca::StepArgs args = a;
+  args.grid_path = 1;  // the step kernel only READS the step counters in this path, from the copy G2 made
+  k.grid<<<(T + tpb - 1) / tpb, tpb, smem, st>>>(args, G.sorted_pv, G.sorted_idx, G.cell_start, G.params, G.env_step_snap,
+                                                 s->d_agent_params);
+  CUDA_TRY(cudaGetLastError());
+  s->launches += orca::kGridLaunchesPerStep;
+  return ORCA_OK;
 }
 
 int launch_step(OrcaSim* s, const orca::StepArgs& a0, int policy, cudaStream_t st) {
@@ -304,21 +314,27 @@ int launch_step(OrcaSim* s, const orca::StepArgs& a0, int policy, cudaStream_t s
     a.nbr_hint = s->d_nbr_hint;  // allocated by orca_create (never inside a launch: the host path captures graphs)
     a.hint_slack = 2.5f * s->p.max_speed * s->p.time_step + 1e-4f;
   }
-  if (s->d_agent_params != nullptr) {
+  if (s->d_agent_params != nullptr)
     a.nd_sq = s->max_nd * s->max_nd;  // what the kernels still read of it: the cell size of the uniform grid
-    const int K = pick_k(s->p.max_neighbors);
-    if (K == 5) return launch_hetero_k<5>(s, a, policy, st);
-    if (K == 10) return launch_hetero_k<10>(s, a, policy, st);
-    return launch_hetero_k<16>(s, a, policy, st);
+  const orca_host::StepPlan p = step_plan_of(s);
+  StepKernels k;
+  switch (policy) {
+    case ORCA_POLICY_EXTERNAL:
+      k = kernels_for<orca::POLICY_EXTERNAL>(p);
+      break;
+    case ORCA_POLICY_GOAL:
+      k = kernels_for<orca::POLICY_GOAL>(p);
+      break;
+    case ORCA_POLICY_RL:
+      k = kernels_for<orca::POLICY_RL>(p);
+      break;
+    case ORCA_POLICY_ALAN:
+      k = kernels_for<orca::POLICY_ALAN>(p);
+      break;
+    default:
+      return fail(ORCA_ERR_INVALID, "unknown policy %d", policy);
   }
-  if (s->N >= s->grid_min_agents) {
-    return orca::launch_grid_step(s->grid, a, policy, st, &s->launches, &g_last_error);
-  }
-  const int k = s->p.max_neighbors;
-  if (k == 5) return launch_small_k<5, true>(s, a, policy, st);
-  if (k == 10) return launch_small_k<10, true>(s, a, policy, st);
-  if (k <= 16) return launch_small_k<16, false>(s, a, policy, st);
-  return fail(ORCA_ERR_UNSUPPORTED, "max_neighbors=%d > 16 is not supported", k);
+  return p.grid ? launch_grid_step(s, a, p, k, st) : launch_tile_step(s, a, p, k, st);
 }
 
 // The largest obstacle range (timeHorizonObst * maxSpeed + radius) of any agent of the handle.
@@ -430,9 +446,9 @@ int ensure_host_staging(OrcaSim* s) {
 }
 
 template <int K>
-int launch_agent_lines(OrcaSim* s, const orca::StepArgs& a, const orca::LinesOut& o, cudaStream_t st) {
+int launch_agent_lines(OrcaSim* s, const orca::StepArgs& a, const orca::LinesOut& o, bool grid, cudaStream_t st) {
   const float4* params = s->d_agent_params;
-  if (s->N >= s->grid_min_agents) {
+  if (grid) {
     // G1-G4 into the query's own grid scratch, without the step-counter bump: nothing a step reads
     // (the step's scratch, the neighbor-search hint, the step counters) is written, so the call needs
     // no ordering against steps -- only against whatever writes pos / vel, and against other
@@ -443,12 +459,8 @@ int launch_agent_lines(OrcaSim* s, const orca::StepArgs& a, const orca::LinesOut
     const int T = s->E * s->N;
     const int tpb = orca::kLinesGridThreads;
     const size_t smem = (size_t)(K + ORCA_MAX_OBST_LINES) * tpb * sizeof(float4);
-    auto kern = orca::agent_lines_grid_kernel<K>;
-    static std::atomic<bool> attr_set[orca::kMaxDevices];  // function attributes are per device
-    if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
-      CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
-    }
+    constexpr auto kern = orca::agent_lines_grid_kernel<K>;
+    CUDA_TRY(set_attrs_once<kern>(s->device, (int)smem, false));
     kern<<<(T + tpb - 1) / tpb, tpb, smem, st>>>(a, G.sorted_pv, G.sorted_idx, G.cell_start, G.params, params, o);
     CUDA_TRY(cudaGetLastError());
     s->launches += orca::kGridLaunchesPerStep;
@@ -459,12 +471,8 @@ int launch_agent_lines(OrcaSim* s, const orca::StepArgs& a, const orca::LinesOut
   args.envs_per_block = tpb / s->N;
   const int blocks = (s->E + args.envs_per_block - 1) / args.envs_per_block;
   const size_t smem = orca::lines_tile_smem_bytes(tpb);
-  auto kern = orca::agent_lines_tile_kernel<K>;
-  static std::atomic<bool> attr_set[orca::kMaxDevices];
-  if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
-    CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
-  }
+  constexpr auto kern = orca::agent_lines_tile_kernel<K>;
+  CUDA_TRY(set_attrs_once<kern>(s->device, (int)smem, false));
   kern<<<blocks, tpb, smem, st>>>(args, params, o);
   CUDA_TRY(cudaGetLastError());
   s->launches += 1;
@@ -485,7 +493,7 @@ int orca_create(const OrcaParams* params, int device, int num_envs, int agents_p
   if (!(params->time_step > 0.f) || !(params->time_horizon > 0.f) || !(params->time_horizon_obst > 0.f))
     return fail(ORCA_ERR_INVALID, "time_step / time_horizon / time_horizon_obst must be > 0");
   if (params->max_neighbors < 0) return fail(ORCA_ERR_INVALID, "max_neighbors must be >= 0");
-  if (pick_k(params->max_neighbors) < 0)
+  if (orca_host::pick_k(params->max_neighbors) < 0)
     return fail(ORCA_ERR_UNSUPPORTED, "max_neighbors=%d > 16 is not supported", params->max_neighbors);
   int ndev = 0;
   CUDA_TRY(cudaGetDeviceCount(&ndev));
@@ -921,10 +929,12 @@ int orca_agent_lines(OrcaSim* s, const float* pos_dev, const float* vel_dev, int
   o.obst_cnt = obst_line_cnt_dev;
   o.max_lines = max_lines;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int K = pick_k(s->p.max_neighbors);
-  if (K == 5) return launch_agent_lines<5>(s, a, o, st);
-  if (K == 10) return launch_agent_lines<10>(s, a, o, st);
-  return launch_agent_lines<16>(s, a, o, st);
+  const bool grid = step_plan_of(s).grid;
+  // pick_k for every handle, uniform ones included: the lines kernels exist for K = 5, 10 and 16 only
+  const int K = orca_host::pick_k(s->p.max_neighbors);
+  if (K == 5) return launch_agent_lines<5>(s, a, o, grid, st);
+  if (K == 10) return launch_agent_lines<10>(s, a, o, grid, st);
+  return launch_agent_lines<16>(s, a, o, grid, st);
 }
 
 int orca_observe(OrcaSim* s, const float* pos_dev, const float* vel_dev, const float* goal_dev, const int32_t* nbr_idx_dev,
@@ -970,14 +980,8 @@ int orca_observe(OrcaSim* s, const float* pos_dev, const float* vel_dev, const f
   const bool paired = orca::obs_table_is_antipodal(a);  // ray i + R / 2 = -ray i: one lane culls for both
   const orca::ObsPlan plan = orca::obs_plan(a, paired);
   const size_t smem = (size_t)plan.warp_bytes * orca::kObsWarps;
-  {
-    static std::atomic<bool> attr_set[orca::kMaxDevices];  // function attributes are per device
-    if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
-      CUDA_TRY(cudaFuncSetAttribute(orca::observe_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-      CUDA_TRY(cudaFuncSetAttribute(orca::observe_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-      if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
-    }
-  }
+  CUDA_TRY(set_attrs_once<orca::observe_kernel<true>>(s->device, 64 * 1024, false));
+  CUDA_TRY(set_attrs_once<orca::observe_kernel<false>>(s->device, 64 * 1024, false));
   const long long per_block = (long long)plan.A * orca::kObsWarps;  // whole agents per warp: their rays share staged data
   const long long blocks = ((long long)s->E * s->N + per_block - 1) / per_block;
   if (paired)
@@ -1018,7 +1022,7 @@ int step_host_route(OrcaSim* s, float* pos_host, float* vel_host, const float* p
   // writes the new positions and velocities into the caller's buffers (as well as into the
   // device-resident state) over PCIe while it computes: no staging copies, no copy-engine
   // start-up per chunk, the transfers overlap the arithmetic warp by warp.  One launch per step.
-  const bool tile_path = s->N < s->grid_min_agents;
+  const bool tile_path = !step_plan_of(s).grid;
   if (tile_path && allow_direct) {
     void *m_pos = nullptr, *m_vel = nullptr, *m_aux = nullptr;
     const bool mapped = cudaHostGetDevicePointer(&m_pos, pos_host, 0) == cudaSuccess &&
@@ -1265,14 +1269,10 @@ int policy_mlp_common(OrcaSim* s, const float* obs_dev, int64_t rows, const Orca
   a.b3 = w->b3_dev;
   a.n_out = w->out_dim;
   a.out = out_dev;
-  static std::atomic<bool> attr_set[orca::kMaxDevices];  // function attributes are per device
   int sm_count = 0;
   CUDA_TRY(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, s->device));
-  if (s->device >= orca::kMaxDevices || !attr_set[s->device].load(std::memory_order_acquire)) {
-    CUDA_TRY(cudaFuncSetAttribute(orca::policy_mlp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)orca::mlp_smem_bytes()));
-    CUDA_TRY(cudaFuncSetAttribute(orca::policy_mlp_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)orca::mlp_tc_smem_bytes()));
-    if (s->device < orca::kMaxDevices) attr_set[s->device].store(true, std::memory_order_release);
-  }
+  CUDA_TRY(set_attrs_once<orca::policy_mlp_kernel>(s->device, (int)orca::mlp_smem_bytes(), false));
+  CUDA_TRY(set_attrs_once<orca::policy_mlp_tc_kernel>(s->device, (int)orca::mlp_tc_smem_bytes(), false));
   if (tensor_cores) {
     const long long tiles = (rows + orca::kTcTile - 1) / orca::kTcTile;
     // persistent: one CTA per SM (195 KB of shared memory), two tile pipelines per CTA

@@ -27,9 +27,7 @@
 #include <cuda_runtime.h>
 #endif
 
-#include <atomic>
 #include <cstdint>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 
@@ -637,67 +635,6 @@ inline int grid_prep(GridScratch& G, const StepArgs& a, int bump, cudaStream_t s
                                                         G.cell_start);
   grid_scatter_kernel<<<nb_agents, tpb, 0, st>>>(a.pos, a.vel, T, G.key, G.slot, G.cell_start, G.sorted_pv, G.sorted_idx);
   return 0;
-}
-
-template <int K, bool KFULL, int POLICY, int OL, bool HETERO = false>
-int launch_grid_kpo(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t* launches, std::string* err,
-                    const float4* agent_params = nullptr) {
-  const int T = a.E * a.N;
-  const int rc = grid_prep(G, a, a.neighbors_only ? 0 : 1, st, err);
-  if (rc != 0) return rc;
-  StepArgs args = a;
-  // the step kernel only READS the step counters in this path, from the copy G2 made
-  const int stpb = ORCA_GRID_TPB;
-  const size_t smem = step_smem_bytes(K, stpb, false, 0, OL, HETERO);
-  auto kern = step_grid_kernel<K, KFULL, POLICY, OL, HETERO>;
-  int dev = 0;
-  ORCA_GRID_TRY(cudaGetDevice(&dev));
-  // function attributes are per device; setting one is idempotent, so a racing second thread is harmless
-  static std::atomic<bool> attr_set[kMaxDevices];
-  if (dev >= kMaxDevices || !attr_set[dev].load(std::memory_order_acquire)) {
-    ORCA_GRID_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ORCA_GRID_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
-    if (dev < kMaxDevices) attr_set[dev].store(true, std::memory_order_release);
-  }
-  args.grid_path = 1;
-  kern<<<(T + stpb - 1) / stpb, stpb, smem, st>>>(args, G.sorted_pv, G.sorted_idx, G.cell_start, G.params, G.env_step_snap, agent_params);
-  ORCA_GRID_TRY(cudaGetLastError());
-  *launches += kGridLaunchesPerStep;
-  return 0;
-}
-
-template <int K, bool KFULL, int POLICY>
-int launch_grid_kp(GridScratch& G, const StepArgs& a, cudaStream_t st, int64_t* launches, std::string* err) {
-  // at most 4 obstacle vertices (none, or one wall): an agent never has more than 2 obstacle lines
-  if (K == 10 && a.world_verts <= 4 && a.vert_stride == 0 && std::getenv("ORCA_B200_NO_SLIM_KERNEL") == nullptr)
-    return launch_grid_kpo<10, true, POLICY, 2>(G, a, st, launches, err);
-  return launch_grid_kpo<K, KFULL, POLICY, ORCA_MAX_OBST_LINES>(G, a, st, launches, err);
-}
-
-template <int K, bool KFULL>
-int launch_grid_k(GridScratch& G, const StepArgs& a, int policy, cudaStream_t st, int64_t* launches, std::string* err) {
-  switch (policy) {
-    case POLICY_EXTERNAL:
-      return launch_grid_kp<K, KFULL, POLICY_EXTERNAL>(G, a, st, launches, err);
-    case POLICY_GOAL:
-      return launch_grid_kp<K, KFULL, POLICY_GOAL>(G, a, st, launches, err);
-    case POLICY_RL:
-      return launch_grid_kp<K, KFULL, POLICY_RL>(G, a, st, launches, err);
-    case POLICY_ALAN:
-      return launch_grid_kp<K, KFULL, POLICY_ALAN>(G, a, st, launches, err);
-    default:
-      *err = "unknown policy";
-      return -1;
-  }
-}
-
-inline int launch_grid_step(GridScratch& G, const StepArgs& a, int policy, cudaStream_t st, int64_t* launches,
-                            std::string* err) {
-  if (a.k == 5) return launch_grid_k<5, true>(G, a, policy, st, launches, err);
-  if (a.k == 10) return launch_grid_k<10, true>(G, a, policy, st, launches, err);
-  if (a.k <= 16) return launch_grid_k<16, false>(G, a, policy, st, launches, err);
-  *err = "max_neighbors > 16 is not supported";
-  return -3;
 }
 
 #endif  // __CUDACC__

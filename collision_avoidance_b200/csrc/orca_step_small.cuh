@@ -21,8 +21,6 @@
 
 namespace orca {
 
-constexpr int kMaxDevices = 64;  // size of the per-device "attribute already set" tables of the launchers
-
 enum : int { POLICY_EXTERNAL = 0, POLICY_GOAL = 1, POLICY_RL = 2, POLICY_ALAN = 3 };
 enum : int { DONE_NONE = 0, DONE_GOAL_RADIUS = 1, DONE_X_BELOW = 2, DONE_GOAL_RADIUS_DEFERRED = 3 };
 enum : int {
